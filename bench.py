@@ -18,6 +18,11 @@ Other workloads (each prints one contract line; the default run reports small ve
                      101-119), global batch 1k / 10k / 100k / 1M split over the N GPUs.
   --workload fm      BASELINE configs[2]: QM9-positional flow-matching training step, batch 512 per GPU.
 --scaling strong splits a fixed global batch over the ranks (default: weak, per-GPU batch fixed).
+--steps sets the number of timed steps of the reported workload (every batch of the sweep).  --dump-outputs DIR writes what
+the last timed step returned as DIR/<name>.npy (float32/float64, at most 64 MB, rows sampled with a fixed seed above that):
+the solve workloads write `samples`, `logs` (log q, log p0(x0), delta), `solver_stats` and `ess_stats`; fm writes the
+updated parameters, EMA, Adam moments, loss and norms.  Inputs and parameters are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 `--impl reference` times the CPU restatement of the reference (oracle/, torch fp32, reverse-mode Jacobian exactly like
 sample_and_log_prob.py:64-66) on the host cores: JAX is not installable in this image, so the reference itself cannot
@@ -208,8 +213,6 @@ def run_reference(args):
     for _ in range(args.steps):
         _, dt = cpu_sample_logq("lj13", params, CPU_TRAJ, threads)
         times.append(dt)
-        if sum(times) > 600.0:       # safety net on a very slow host only: K x ~14 s fits on the 16-core boxes (K = 20 -> 272 s)
-            break
     value = CPU_TRAJ * len(times) / sum(times)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -256,6 +259,26 @@ def count_kernels(fn):
         return ours, others, names
     except Exception as e:  # noqa: BLE001
         return None, None, {"error": repr(e)}
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Writes `arrays` (what the timed path returned in its last step) as <path>/<name>.npy in float32 or float64, so that
+    two builds can be compared output for output.  Integer outputs become float64 (exact).  When the whole exceeds 64 MB,
+    every array keeps the same fixed, seeded sample of its rows."""
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        host[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in host.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in host.items():
+        if total > DUMP_MAX_BYTES and a.ndim > 0 and a.shape[0] > 1:
+            keep = max(1, a.shape[0] * DUMP_MAX_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class Ctx:
@@ -375,7 +398,9 @@ def bench_solve(c, name: str, b_begin: int, b_end: int, *, div: bool, adaptive: 
     k_ms = sum(a.elapsed_time(b) for a, b in kernel_events) / len(kernel_events)
     out = {"value": global_B * steps / (total_ms * 1e-3), "ms_per_step": total_ms / steps, "kernel_ms": k_ms,
            "evals_per_launch": evals_last, "batch_this_rank": B, "global_batch": global_B, "step_ms": t_steps,
-           "clocks": clocks, "status_failures": bad, "eng": eng, "D": D}
+           "clocks": clocks, "status_failures": bad, "eng": eng, "D": D,
+           "outputs": {k: v for k, v in (("samples", x1), ("logs", logs), ("solver_stats", stats), ("ess_stats", st))
+                       if v is not None}}
     if st is not None:
         rv, fw = ess_from_stats(st.tolist(), global_B)
         out["reverse_ess"], out["forward_ess"] = rv, fw
@@ -497,6 +522,10 @@ def bench_train(c, *, steps: int = 10, cpu: bool = False, chunk: int = 0, count:
         barrier(c)
         res[label] = max_over_ranks(c, a.elapsed_time(b)) / steps
     loss = float(info["loss"])
+    # copies: the launch-count step below updates the donated buffers in place
+    outputs = {"params": state.params.flat, "ema_params": state.ema_params.flat, "adam_mu": state.opt_state.mu,
+               "adam_nu": state.opt_state.nu, **info}
+    outputs = {k: v.clone() for k, v in outputs.items()}
     holder = {"s": state}
 
     def one():
@@ -513,7 +542,8 @@ def bench_train(c, *, steps: int = 10, cpu: bool = False, chunk: int = 0, count:
                    "d2h_bytes_per_step": 4, "note": "+ a device->host read of the loss every step"},
            "roofline": {"bound": "tensor", "achieved": tf, "peak": peak, "unit": "TFLOP/s", "frac": tf / peak,
                         "algorithmic_flops_per_step": flops, "per": "GPU", "peak_source": f"{pk_kind} bf16 dense burst"},
-           "kernels_per_step": {"ours": ours, "torch_or_library": others}, "launches_per_step": ours or 1}
+           "kernels_per_step": {"ours": ours, "torch_or_library": others}, "launches_per_step": ours or 1,
+           "outputs": outputs}
     if cpu and c.rank == 0 and c.world == 1:
         threads = os.cpu_count() or 1
         v, dt, l_cpu = cpu_fm_steps(B, 3, threads)
@@ -538,7 +568,7 @@ def contract_line(c, args, *, metric, unit, r, workload, cfg_extra, roofline, cp
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 2; 10 for --workload fm)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="lj13", choices=["lj13", "aldp", "dw4", "sweep", "fm"])
@@ -550,7 +580,13 @@ def main():
     ap.add_argument("--sweep-max", type=int, default=1_000_000)
     ap.add_argument("--fm-chunk", type=int, default=0, help="fm workload: graphs per chunk of the minibatch (0 = automatic)")
     ap.add_argument("--no-count", action="store_true", help="skip the profiler pass that counts kernel launches (one extra step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (rank 0's shard under torchrun)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 10 if args.workload == "fm" else 2
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         return run_reference(args)
     c = setup(args)
@@ -667,14 +703,13 @@ def main():
             if gb > args.sweep_max:
                 continue
             b0, b1 = shard(c, gb)
-            nsteps = 1 if gb >= 100_000 else args.steps
-            # (the kernel and its workspace are warm after the smaller batches: the long ones are timed once, without a warm-up pass)
-            r = bench_solve(c, "lj13", b0, b1, div=False, adaptive=args.adaptive, steps=nsteps,
+            # (the kernel and its workspace are warm after the smaller batches: the long ones are timed without a warm-up pass)
+            r = bench_solve(c, "lj13", b0, b1, div=False, adaptive=args.adaptive, steps=args.steps,
                             warmup=1 if gb <= 10_000 else 0, target=None, e2e_steps=1 if gb <= 10_000 else 0,
                             count=(gb == 1_000 and not args.no_count))
             if gb == 1_000:
                 per_step = r["launches_per_step"]
-            total_launches += per_step * nsteps
+            total_launches += per_step * args.steps
             table.append({"global_batch": gb, "samples_per_s": r["value"], "ms": r["ms_per_step"],
                           "e2e_samples_per_s": r["e2e"]["value"] if "e2e" in r else None,
                           "roofline_frac": roofline_of(c, "lj13", r, False)["frac"]})
@@ -696,19 +731,22 @@ def main():
                              launches=total_launches)
 
     elif args.workload == "fm":
-        ft = bench_train(c, steps=max(args.steps, 10), cpu=not args.no_cpu, chunk=args.fm_chunk, count=not args.no_count)
+        ft = bench_train(c, steps=args.steps, cpu=not args.no_cpu, chunk=args.fm_chunk, count=not args.no_count)
         line = {"metric": ft["metric"], "value": ft["value"], "unit": "steps/s", "n_gpus": c.world,
-                "steps": max(args.steps, 10), "warmup": 3, "ms_per_step": ft["ms_per_step"], "higher_is_better": True,
+                "steps": args.steps, "warmup": 3, "ms_per_step": ft["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                 "config": {"workload": "qm9pos_flow_matching_update_fn_batch512_per_gpu", "global_batch": ft["global_batch"],
                            "parallelism": f"dp{c.world} (minibatch shards, one NCCL all-reduce of the flat gradient)"},
                 "roofline": ft["roofline"], "cpu_baseline": ft.get("cpu_baseline"), "e2e": ft["e2e"],
-                "gpu_launches": ft["launches_per_step"] * max(args.steps, 10), "extra": {"loss": ft["loss"], "kernels_per_step": ft["kernels_per_step"], "fm_chunk": args.fm_chunk}}
+                "gpu_launches": ft["launches_per_step"] * args.steps, "extra": {"loss": ft["loss"], "kernels_per_step": ft["kernels_per_step"], "fm_chunk": args.fm_chunk}}
 
+    if args.dump_outputs and c.rank == 0:
+        headline = ft if args.workload == "fm" else last if args.workload == "sweep" else r
+        dump_outputs(args.dump_outputs, headline["outputs"])
     if c.rank == 0:
         def clean(o):
             if isinstance(o, dict):
-                return {k: clean(v) for k, v in o.items() if k != "eng"}
+                return {k: clean(v) for k, v in o.items() if k not in ("eng", "outputs")}
             if isinstance(o, list):
                 return [clean(v) for v in o]
             return o

@@ -4,6 +4,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 import bench
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -25,6 +28,27 @@ def test_reference_arm_is_silent_on_other_ranks():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                        capture_output=True, text=True, env=env, timeout=120)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_floats_and_a_fixed_sample_above_the_cap(tmp_path, monkeypatch):
+    stats = torch.arange(40, dtype=torch.int32).reshape(10, 4)
+    outputs = {"samples": torch.randn(10, 3), "solver_stats": stats, "loss": torch.tensor(1.5, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "all"), outputs)
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").iterdir()}
+    assert set(got) == set(outputs)
+    assert got["samples"].dtype == np.float32 and np.array_equal(got["samples"], outputs["samples"].numpy())
+    assert got["solver_stats"].dtype == np.float64 and np.array_equal(got["solver_stats"], stats.numpy())
+    assert got["loss"].shape == () and float(got["loss"]) == 1.5
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 256)              # 10 x 3 x 4 + 10 x 4 x 8 + 8 = 448 bytes in all
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), outputs)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    b = {p.stem: np.load(p) for p in (tmp_path / "b").iterdir()}
+    assert sum(v.nbytes for v in a.values()) <= 256
+    rows = [np.flatnonzero((got["solver_stats"] == r).all(axis=1))[0] for r in a["solver_stats"]]
+    assert len(rows) == 5 and rows == sorted(rows)                  # the same rows of every array, in order
+    assert np.array_equal(a["samples"], got["samples"][rows])
+    assert all(np.array_equal(a[k], b[k]) for k in a)
 
 
 def test_cpu_arm_builds_its_parameters_without_the_cuda_library():
