@@ -16,6 +16,16 @@ int launch_uh(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st) {
   return ECNF_ERR_UNSUPPORTED;
 }
 
+template <bool DIV>
+int simt_check_uh(const ecnf_model* mdl) {
+  const int U = mdl->cfg.mlp_units, H = mdl->cfg.n_hidden;
+  if (U == 128 && H == 64) return simt_check<128, 64, DIV>(mdl);
+  if (U == 256 && H == 32) return simt_check<256, 32, DIV>(mdl);
+  if (U == 64 && H == 32) return simt_check<64, 32, DIV>(mdl);
+  ecnf_set_error("unsupported (mlp_units=%d, n_hidden=%d): compiled pairs are (128,64), (256,32), (64,32)", U, H);
+  return ECNF_ERR_UNSUPPORTED;
+}
+
 int grid_for(const ecnf_model* m, int64_t B) {
   int64_t g = m->num_sms;
   if (B < g) g = B;
@@ -90,6 +100,17 @@ int64_t ecnf_solve_workspace_bytes(const ecnf_model* m, int mode, int64_t B) {
 int64_t ecnf_solve_tensor_flops_per_eval(const ecnf_model* m) {
   if (!m || !use_tc(m, true)) return 0;
   return tc_flops_per_eval(m);
+}
+
+int ecnf_solve_engine_for(const ecnf_model* m, int mode) {
+  if (!m || mode < ECNF_MODE_VF || mode > ECNF_MODE_LOGPROB) {
+    ecnf_set_error("ecnf_solve_engine_for: null model or bad mode %d", mode);
+    return ECNF_ERR_INVALID;
+  }
+  const bool div = mode_div(mode);
+  if (use_tc(m, div)) return 0;
+  const int rc = div ? simt_check_uh<true>(m) : simt_check_uh<false>(m);
+  return rc == ECNF_OK ? 1 : rc;
 }
 
 int ecnf_solve_tc_tile_table(const ecnf_model* m, int kind, uint32_t* out_host, int64_t cap_words) {

@@ -55,6 +55,9 @@ struct KernelArgs {
   TcTabs tabs;
 };
 
+// fp32 SIMT engine: its shape limits (ECNF_OK, or ECNF_ERR_UNSUPPORTED with the reason set), launch
+template <int U, int H, bool DIV>
+int simt_check(const ecnf_model* mdl);
 template <int U, int H, bool DIV>
 int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st);
 

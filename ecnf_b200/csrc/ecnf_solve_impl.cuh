@@ -841,7 +841,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ecnf_solve_kernel(const __grid_co
 }
 
 template <int U, int H, bool DIV>
-int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st) {
+int simt_check(const ecnf_model* mdl) {
   const SmemLayout L = make_layout<U, H>(mdl->cfg.n_frames, mdl->cfg.dim, DIV);
   const size_t smem = (size_t)L.total_floats * sizeof(float);
   if (smem > 227 * 1024) {
@@ -854,6 +854,14 @@ int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st) {
                    Geo<U, H>::TR, U);
     return ECNF_ERR_UNSUPPORTED;
   }
+  return ECNF_OK;
+}
+
+template <int U, int H, bool DIV>
+int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st) {
+  const int rc = simt_check<U, H, DIV>(mdl);
+  if (rc != ECNF_OK) return rc;
+  const size_t smem = (size_t)make_layout<U, H>(mdl->cfg.n_frames, mdl->cfg.dim, DIV).total_floats * sizeof(float);
   auto kern = ecnf_solve_kernel<U, H, DIV>;
   ECNF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, NTHREADS, smem, st>>>(a);

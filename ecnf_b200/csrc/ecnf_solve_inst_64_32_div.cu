@@ -2,4 +2,5 @@
 #include "ecnf_solve_impl.cuh"
 namespace ecnf_solve_detail {
 template int launch_t<64, 32, true>(const ecnf_model*, KernelArgs&, int, cudaStream_t);
+template int simt_check<64, 32, true>(const ecnf_model*);
 }

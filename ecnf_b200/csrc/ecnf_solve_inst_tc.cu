@@ -1,4 +1,5 @@
 // Tensor-core (tcgen05 / TMEM) instantiations of engine A + their weight-image / tile-table preparation.
+#include <algorithm>
 #include <vector>
 
 #include "ecnf_solve_tc.cuh"
@@ -21,16 +22,14 @@ TcSmemLayout layout_of(const ecnf_config& c, int MR) {
   return c.mlp_units == 128 ? make_tc_layout<128, 64>(c.n_frames, c.dim, MR) : make_tc_layout<64, 32>(c.n_frames, c.dim, MR);
 }
 
-// walks the images in a fixed order; fills the offsets and (optionally) the prep list
-int64_t walk_images(const ecnf_model* mdl, TcImages* img, TcPrepList* list) {
+// walks the images (3 L + 3 per block) in a fixed order; fills the offsets and (optionally) the prep items
+int64_t walk_images(const ecnf_model* mdl, TcImages* img, std::vector<TcPrepItem>* items) {
   const ecnf_config& c = mdl->cfg;
   const int H = c.n_hidden, U = c.mlp_units, L = c.n_layers, SUB = sub_of(c);
   int64_t off = 0;
-  int cnt = 0;
   auto add = [&](int64_t src_off, int ksub, int N) {
     const int64_t o = off;
-    if (list && cnt < 64) list->item[cnt] = TcPrepItem{(int)src_off, (int)o, ksub, N, SUB, U};
-    ++cnt;
+    if (items) items->push_back(TcPrepItem{(int)src_off, (int)o, ksub, N, SUB, U});
     off += (int64_t)(SUB * ksub) * 512;   // hi | lo, 128 lanes x K/2 words each
     return (int)o;
   };
@@ -47,7 +46,6 @@ int64_t walk_images(const ecnf_model* mdl, TcImages* img, TcPrepList* list) {
     ib.WhL = add(po.Wh[L], U, H);
     if (img) img->blk[b] = ib;
   }
-  if (list) list->count = cnt;
   return off;
 }
 
@@ -133,16 +131,18 @@ int tc_tile_table(const ecnf_model* mdl, int kind, uint32_t* out, int64_t cap_wo
 
 int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bool div, cudaStream_t st) {
   const ecnf_config& c = mdl->cfg;
-  TcPrepList local{};
+  std::vector<TcPrepItem> items;
   a.img.base = reinterpret_cast<const unsigned char*>(image_ws);
-  walk_images(mdl, &a.img, &local);
-  if (local.count > 64) {
-    ecnf_set_error("tensor-core path: %d weight images exceed the prep list", local.count);
-    return ECNF_ERR_UNSUPPORTED;
+  walk_images(mdl, &a.img, &items);
+  // up to 8 blocks x (3 L + 3) = 168 images: one prep launch per slice of at most TC_PREP_MAX of them
+  for (size_t i0 = 0; i0 < items.size(); i0 += TC_PREP_MAX) {
+    TcPrepList list{};
+    list.count = (int)std::min(items.size() - i0, (size_t)TC_PREP_MAX);
+    std::copy(items.begin() + i0, items.begin() + i0 + list.count, list.item);
+    dim3 pgrid(16, list.count);
+    tc_prep_kernel<<<pgrid, 256, 0, st>>>(mdl->d_params, reinterpret_cast<unsigned char*>(image_ws), list);
+    ECNF_CHECK_CUDA(cudaGetLastError());
   }
-  dim3 pgrid(16, local.count);
-  tc_prep_kernel<<<pgrid, 256, 0, st>>>(mdl->d_params, reinterpret_cast<unsigned char*>(image_ws), local);
-  ECNF_CHECK_CUDA(cudaGetLastError());
   const int MR = pick_mrows(c, div);
   // Hutchinson (a.eps given): one tangent direction -- the tables of kinds TT_NODE / TT_MID with two rows per group
   const int ntan = (div && a.eps) ? 1 : c.n_frames * c.dim;

@@ -1454,9 +1454,10 @@ struct TcPrepItem {
   int ksub, N;   // rows / columns of the source matrix
   int nsub, lane_stride;
 };
+constexpr int TC_PREP_MAX = 64;   // items per tc_prep_kernel launch (the list is a by-value kernel parameter)
 struct TcPrepList {
   int count;
-  TcPrepItem item[64];
+  TcPrepItem item[TC_PREP_MAX];
 };
 
 __global__ void tc_prep_kernel(const float* __restrict__ params, unsigned char* __restrict__ image, const TcPrepList list) {

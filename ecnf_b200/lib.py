@@ -64,6 +64,7 @@ SIGNATURES = {
     "ecnf_model_set_engine": (C.c_int, [_P, C.c_int]),
     "ecnf_model_set_fm_chunk": (C.c_int, [_P, C.c_int64]),
     "ecnf_solve_tensor_flops_per_eval": (C.c_int64, [C.c_void_p]),
+    "ecnf_solve_engine_for": (C.c_int, [_P, C.c_int]),
     "ecnf_solve_tc_tile_table": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.c_int64]),
     "ecnf_vf_forward": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _I64, _P]),
     "ecnf_vf_forward_div": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I64, _P]),

@@ -84,6 +84,11 @@ int ecnf_model_set_engine(ecnf_model* m, int engine);
 /* tcgen05 flops the tensor-core engine issues per vector-field evaluation with exact divergence (3 bf16 passes over
  * every 128-lane x N-column tile-layer), 0 when the shape runs on the fp32 SIMT engine.  For roofline reports.   */
 int64_t ecnf_solve_tensor_flops_per_eval(const ecnf_model* m);
+/* Which engine a solve / vector-field call of `mode` (ECNF_MODE_*; VF_DIV covers the Hutchinson entry points too) runs on
+ * with this handle's current engine choice: 0 = tcgen05 tensor cores, 1 = fp32 SIMT; negative = that call would fail
+ * (ECNF_ERR_UNSUPPORTED: the shape exceeds the SIMT engine's limits, ecnf_last_error() says which; ECNF_ERR_INVALID: null
+ * handle or bad mode).  No device work.                                                                             */
+int ecnf_solve_engine_for(const ecnf_model* m, int mode);
 /* Host copy of the tensor-core engine's tile table of one kind (0 node/primal-only, 1 node, 2 first-block edges,
  * 3 middle-block edges, 4 last-block edges, 5 edges/primal-only; kind + 8: the one-tangent (Hutchinson) variant, used for
  * kinds 1 and 3): 48 uint32 per tile = 32 chunk words (2 sub-tiles x 16 chunks of 8 columns: bit31 valid, [0,10) group,
