@@ -64,6 +64,20 @@ __device__ __forceinline__ float fast_sigmoid(float z) {
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.f + e));
   return r;
 }
+// the same on a pair (the two multiplies and adds packed, ex2 / rcp per lane)
+__device__ __forceinline__ float2 fast_sigmoid2(float2 z) {
+  const float2 t = mul2(z, splat2(-1.4426950408889634f));
+  float2 e, r;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.x) : "f"(t.x));
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.y) : "f"(t.y));
+  const float2 d = add2(splat2(1.f), e);
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r.x) : "f"(d.x));
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r.y) : "f"(d.y));
+  return r;
+}
+// columns (c, c + 1) of a thread's 64 accumulator values as a pair (c even)
+__device__ __forceinline__ float2 col2(const float (&v)[64], int c) { return make_float2(v[c], v[c + 1]); }
+__device__ __forceinline__ void set_col2(float (&v)[64], int c, float2 p) { v[c] = p.x; v[c + 1] = p.y; }
 
 // ntan = tangent directions carried: n * dim (exact trace: the basis) or 1 (Hutchinson: the probe; tables TT_NODE and TT_MID)
 __host__ __device__ inline int tc_rows_of_kind(int kind, int n, int dim, int ntan) {
@@ -456,30 +470,7 @@ struct EngineTC {
   __device__ __forceinline__ void act_half(float (&v)[64], int hf, float bias, int tb, float wdf) {
     const float* sdp = TCF(colsd) + (tb * SUB + sub) * 128 + 64 * hh;
 #pragma unroll
-    for (int c4 = 0; c4 < 4; ++c4) {
-      const int ch = 4 * hf + c4;
-      if constexpr (L0) {
-        const float4 s0 = reinterpret_cast<const float4*>(sdp)[2 * ch], s1 = reinterpret_cast<const float4*>(sdp)[2 * ch + 1];
-        v[8 * ch] = fmaf(s0.x, wdf, v[8 * ch]); v[8 * ch + 1] = fmaf(s0.y, wdf, v[8 * ch + 1]);
-        v[8 * ch + 2] = fmaf(s0.z, wdf, v[8 * ch + 2]); v[8 * ch + 3] = fmaf(s0.w, wdf, v[8 * ch + 3]);
-        v[8 * ch + 4] = fmaf(s1.x, wdf, v[8 * ch + 4]); v[8 * ch + 5] = fmaf(s1.y, wdf, v[8 * ch + 5]);
-        v[8 * ch + 6] = fmaf(s1.z, wdf, v[8 * ch + 6]); v[8 * ch + 7] = fmaf(s1.w, wdf, v[8 * ch + 7]);
-      }
-      if constexpr (!DIV) {      // every column is a primal row
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const float z = v[8 * ch + u] + bias;
-          v[8 * ch + u] = z * fast_sigmoid(z);
-        }
-      } else {
-        const float z = v[8 * ch] + bias;
-        const float sg = fast_sigmoid(z);
-        const float cur = sg * (1.f + z * (1.f - sg));
-        v[8 * ch] = z * sg;
-#pragma unroll
-        for (int u = 1; u < 8; ++u) v[8 * ch + u] *= cur;
-      }
-    }
+    for (int c4 = 0; c4 < 4; ++c4) act_chunk<L0>(v, 4 * hf + c4, bias, sdp, wdf);
   }
   __device__ __forceinline__ void write_half(int s, const float (&v)[64], int hf, int krow) {
     unsigned char* base = smem_tc + a.lay.bop + s * TC_BOP + (8 * hh + 4 * hf) * (int)TC_SBO + krow * 16;
@@ -505,28 +496,34 @@ struct EngineTC {
   __device__ __forceinline__ void act_rule(float (&v)[64], float bias, int tb, float wdf) {
     const float* sdp = TCF(colsd) + (tb * SUB + sub) * 128 + 64 * hh;
 #pragma unroll
-    for (int ch = 0; ch < 8; ++ch) {
-      if constexpr (L0) {
-        const float4 s0 = reinterpret_cast<const float4*>(sdp)[2 * ch], s1 = reinterpret_cast<const float4*>(sdp)[2 * ch + 1];
-        v[8 * ch] = fmaf(s0.x, wdf, v[8 * ch]); v[8 * ch + 1] = fmaf(s0.y, wdf, v[8 * ch + 1]);
-        v[8 * ch + 2] = fmaf(s0.z, wdf, v[8 * ch + 2]); v[8 * ch + 3] = fmaf(s0.w, wdf, v[8 * ch + 3]);
-        v[8 * ch + 4] = fmaf(s1.x, wdf, v[8 * ch + 4]); v[8 * ch + 5] = fmaf(s1.y, wdf, v[8 * ch + 5]);
-        v[8 * ch + 6] = fmaf(s1.z, wdf, v[8 * ch + 6]); v[8 * ch + 7] = fmaf(s1.w, wdf, v[8 * ch + 7]);
-      }
-      if constexpr (!DIV) {      // every column is a primal row
+    for (int ch = 0; ch < 8; ++ch) act_chunk<L0>(v, ch, bias, sdp, wdf);
+  }
+  // the rule on chunk ch, on column pairs (every lane of a pair is the scalar operation of that column):
+  // the primal column's z * sigmoid(z) shares its multiply with column 1's tangent scaling
+  template <bool L0>
+  __device__ __forceinline__ static void act_chunk(float (&v)[64], int ch, float bias, const float* sdp, float wdf) {
+    const int c0 = 8 * ch;
+    if constexpr (L0) {      // z += |v|^2 w_d
+      const float4 s0 = reinterpret_cast<const float4*>(sdp)[2 * ch], s1 = reinterpret_cast<const float4*>(sdp)[2 * ch + 1];
+      const float2 w2 = splat2(wdf);
+      set_col2(v, c0, fma2(make_float2(s0.x, s0.y), w2, col2(v, c0)));
+      set_col2(v, c0 + 2, fma2(make_float2(s0.z, s0.w), w2, col2(v, c0 + 2)));
+      set_col2(v, c0 + 4, fma2(make_float2(s1.x, s1.y), w2, col2(v, c0 + 4)));
+      set_col2(v, c0 + 6, fma2(make_float2(s1.z, s1.w), w2, col2(v, c0 + 6)));
+    }
+    if constexpr (!DIV) {      // every column is a primal row
 #pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const float z = v[8 * ch + u] + bias;
-          v[8 * ch + u] = z * fast_sigmoid(z);
-        }
-      } else {
-        const float z = v[8 * ch] + bias;
-        const float sg = fast_sigmoid(z);
-        const float cur = sg * (1.f + z * (1.f - sg));
-        v[8 * ch] = z * sg;
-#pragma unroll
-        for (int u = 1; u < 8; ++u) v[8 * ch + u] *= cur;
+      for (int u = 0; u < 8; u += 2) {
+        const float2 z = add2(col2(v, c0 + u), splat2(bias));
+        set_col2(v, c0 + u, mul2(z, fast_sigmoid2(z)));
       }
+    } else {
+      const float z = v[c0] + bias;
+      const float sg = fast_sigmoid(z);
+      const float cur = sg * (1.f + z * (1.f - sg));
+      set_col2(v, c0, mul2(make_float2(z, v[c0 + 1]), make_float2(sg, cur)));
+#pragma unroll
+      for (int u = 2; u < 8; u += 2) set_col2(v, c0 + u, mul2(col2(v, c0 + u), splat2(cur)));
     }
   }
   template <int W>   // 2W partial sums -> W, exchanging with lane ^ (W/2)
@@ -544,11 +541,16 @@ struct EngineTC {
     float x[32];
     {
       const bool b = (lane & 16) != 0;
+      const float2 w2 = splat2(wf);
 #pragma unroll
-      for (int i = 0; i < 32; ++i) {
-        const float lo = v[i] * wf, hi = v[32 + i] * wf;
-        const float keep = b ? hi : lo, send = b ? lo : hi;
-        x[i] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
+      for (int i = 0; i < 32; i += 2) {
+        const float2 lo2 = mul2(col2(v, i), w2), hi2 = mul2(col2(v, 32 + i), w2);
+        const float lo[2] = {lo2.x, lo2.y}, hi[2] = {hi2.x, hi2.y};
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const float keep = b ? hi[j] : lo[j], send = b ? lo[j] : hi[j];
+          x[i + j] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
+        }
       }
     }
     bfly_round<16>(x);
@@ -1281,19 +1283,19 @@ struct EngineTC {
       } else {
         const float* wb_ = TCF(wB) + warp * 64;
         const float inv_sqrt_nb = rsqrtf((float)(e.n - 1));
-        float acc[8];
+        float2 acc2[4];      // columns (2k, 2k + 1) of the chunk: acc = v wa + (curm wb + acc), per lane as fmaf(v, wa, fmaf(curm, wb, acc))
 #pragma unroll
-        for (int u = 0; u < 8; ++u) acc[u] = 0.f;
+        for (int k = 0; k < 4; ++k) acc2[k] = make_float2(0.f, 0.f);
 #pragma unroll
         for (int ch = 0; ch < 8; ++ch) {
           if (ch < nc) {
-            const float curm = v[8 * ch];
+            const float2 curm = splat2(v[8 * ch]);
             const float4 wa0 = reinterpret_cast<const float4*>(wa_)[2 * ch], wa1 = reinterpret_cast<const float4*>(wa_)[2 * ch + 1];
             const float4 wb0 = reinterpret_cast<const float4*>(wb_)[2 * ch], wb1 = reinterpret_cast<const float4*>(wb_)[2 * ch + 1];
-            const float wav[8] = {wa0.x, wa0.y, wa0.z, wa0.w, wa1.x, wa1.y, wa1.z, wa1.w};
-            const float wbv[8] = {wb0.x, wb0.y, wb0.z, wb0.w, wb1.x, wb1.y, wb1.z, wb1.w};
+            const float2 wav[4] = {make_float2(wa0.x, wa0.y), make_float2(wa0.z, wa0.w), make_float2(wa1.x, wa1.y), make_float2(wa1.z, wa1.w)};
+            const float2 wbv[4] = {make_float2(wb0.x, wb0.y), make_float2(wb0.z, wb0.w), make_float2(wb1.x, wb1.y), make_float2(wb1.z, wb1.w)};
 #pragma unroll
-            for (int u = 0; u < 8; ++u) acc[u] = fmaf(v[8 * ch + u], wav[u], fmaf(curm, wbv[u], acc[u]));
+            for (int k = 0; k < 4; ++k) acc2[k] = fma2(col2(v, 8 * ch + 2 * k), wav[k], fma2(curm, wbv[k], acc2[k]));
             if (e.my_chw(tb, ch) & CH_GRPEND) {
               // my last chunk of this run: add the run's partial sums to the accumulator rows of its columns (distinct rows;
               // padding shares the dump row); a negative entry is a per-sender row of the first block, stored straight to M
@@ -1303,10 +1305,17 @@ struct EngineTC {
 #pragma unroll
               for (int u = 0; u < 8; ++u) old[u] = mac[mr[u] >= 0 ? mr[u] : a.lay.mrows * U];
 #pragma unroll
-              for (int u = 0; u < 8; ++u) {
-                if (mr[u] >= 0) mac[mr[u]] = old[u] + acc[u];
-                else e.Mg()[(size_t)(-1 - mr[u]) * U + e.fu] = acc[u] * inv_sqrt_nb;
-                acc[u] = 0.f;
+              for (int k = 0; k < 4; ++k) {
+                const float acc[2] = {acc2[k].x, acc2[k].y};
+                const float2 sum = add2(make_float2(old[2 * k], old[2 * k + 1]), acc2[k]);
+                const float s[2] = {sum.x, sum.y};
+#pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                  const int u = 2 * k + j;
+                  if (mr[u] >= 0) mac[mr[u]] = s[j];
+                  else e.Mg()[(size_t)(-1 - mr[u]) * U + e.fu] = acc[j] * inv_sqrt_nb;
+                }
+                acc2[k] = make_float2(0.f, 0.f);
               }
             }
           }

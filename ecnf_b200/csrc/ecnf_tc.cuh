@@ -179,12 +179,45 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8])
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+// ---- packed fp32 pairs: one FFMA2 / FMUL2 / FADD2 does the two IEEE round-to-nearest operations of the scalar
+// instructions it replaces (bit for bit), in one issue slot.  nvcc does not pair scalar code by itself. -------------------
+__device__ __forceinline__ float2 fma2(float2 x, float2 y, float2 z) {    // (fmaf(x.x, y.x, z.x), fmaf(x.y, y.y, z.y))
+  float2 d;
+  asm("{\n\t.reg .b64 a, b, c, d;\n\t"
+      "mov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tmov.b64 c, {%6, %7};\n\t"
+      "fma.rn.f32x2 d, a, b, c;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(d.x), "=f"(d.y)
+      : "f"(x.x), "f"(x.y), "f"(y.x), "f"(y.y), "f"(z.x), "f"(z.y));
+  return d;
+}
+__device__ __forceinline__ float2 mul2(float2 x, float2 y) {
+  float2 d;
+  asm("{\n\t.reg .b64 a, b, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tmul.rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(d.x), "=f"(d.y) : "f"(x.x), "f"(x.y), "f"(y.x), "f"(y.y));
+  return d;
+}
+__device__ __forceinline__ float2 add2(float2 x, float2 y) {
+  float2 d;
+  asm("{\n\t.reg .b64 a, b, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tadd.rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(d.x), "=f"(d.y) : "f"(x.x), "f"(x.y), "f"(y.x), "f"(y.y));
+  return d;
+}
+__device__ __forceinline__ float2 sub2(float2 x, float2 y) {
+  float2 d;
+  asm("{\n\t.reg .b64 a, b, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tsub.rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(d.x), "=f"(d.y) : "f"(x.x), "f"(x.y), "f"(y.x), "f"(y.y));
+  return d;
+}
+__device__ __forceinline__ float2 splat2(float x) { return make_float2(x, x); }
+
 // ---- fp32 -> (hi, lo) bf16 split of two consecutive K elements, packed for a TMEM column (low half = even k) -------
+// hi = round-to-nearest bf16 of x; lo = the same rounding of the exact residual x - float(hi).  The two halves of the
+// packed hi word are widened back to fp32 by a shift and a mask (bf16 is the top half of an fp32).
 __device__ __forceinline__ void split_pack(float x0, float x1, uint32_t& hi, uint32_t& lo) {
   const __nv_bfloat162 h = __floats2bfloat162_rn(x0, x1);      // .x = x0 (low 16 bits), .y = x1
-  const float r0 = x0 - __low2float(h), r1 = x1 - __high2float(h);
-  const __nv_bfloat162 l = __floats2bfloat162_rn(r0, r1);
   hi = *reinterpret_cast<const uint32_t*>(&h);
+  const float2 r = sub2(make_float2(x0, x1), make_float2(__uint_as_float(hi << 16), __uint_as_float(hi & 0xffff0000u)));
+  const __nv_bfloat162 l = __floats2bfloat162_rn(r.x, r.y);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
