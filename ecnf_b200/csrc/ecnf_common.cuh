@@ -49,7 +49,7 @@ struct ecnf_model {
   int num_sms;
   int device;
   int engine;   // ecnf_model_set_engine: 0 = tensor cores where eligible, 1 = fp32 SIMT everywhere
-  int64_t fm_chunk;   // ecnf_model_set_fm_chunk: graphs per chunk of a training minibatch, 0 = automatic
+  int64_t fm_chunk;   // ecnf_model_set_fm_chunk: graphs per chunk of a training minibatch, 0 = the whole minibatch
 };
 
 EcnfModelDev ecnf_make_dev(const ecnf_model* m, const float* d_params);

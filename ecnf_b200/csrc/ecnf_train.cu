@@ -6,8 +6,9 @@
 //
 // Layout in HBM: every Dense layer is one row-major [rows x width] fp32 matrix over the whole batch, rows =
 // B*n node rows or B*n*(n-1) edge rows (receiver-major inside a graph, utils/graph.py:6-14).  The forward keeps
-// the pre-activations z of every layer; the backward overwrites them in place with dz.  GEMMs use the same
-// register-tiled fp32 building block as engine A (ecnf_tile.cuh).
+// the pre-activations z of every layer; the backward overwrites them in place with dz.  The square GEMMs and weight
+// gradients over the edge rows run on the tensor cores (ecnf_train_tc.cuh); every other GEMM, and all of them when the
+// handle selects the SIMT engine, uses the register-tiled fp32 building block of engine A (ecnf_tile.cuh).
 #include <algorithm>
 
 #include "ecnf_tile.cuh"
@@ -18,10 +19,22 @@ using ecnf_tile::ColT;
 using ecnf_tile::NTHREADS;
 using ecnf_tile::tile_gemm;
 using ecnf_tile::WCHUNK;
+using ecnf_train_tc::GemmArgs;
 
-// engine choice of the model handle of the ecnf_fm_loss_grad call running on this host thread (0 = tensor cores where
-// eligible, 1 = fp32 SIMT): read once at entry, so concurrent callers with different handles do not interfere
-thread_local int t_engine = 0;
+// What every launch of one ecnf_fm_loss_grad call needs from the model handle and the caller
+struct LaunchCtx {
+  int num_sms;
+  bool use_tc;   // the handle's engine choice: tensor cores where eligible (engine 0), or fp32 SIMT everywhere
+  cudaStream_t st;
+};
+
+// Shapes with a tensor-core kernel (ecnf_train_tc.cuh)
+constexpr bool tc_shape(int K, int N) { return K == N && (K == 128 || K == 256); }
+// The big square GEMMs over the edge rows go to the tensor cores.  `plain`: dense leading dimensions, no second operand
+// and no per-graph row vector, which only the SIMT kernels support.
+bool use_tc(const LaunchCtx& lc, int K, int N, int M, bool plain) {
+  return lc.use_tc && plain && tc_shape(K, N) && M >= 8192;
+}
 
 __device__ __forceinline__ float silu_f(float z) { return z * ecnf_sigmoid(z); }
 __device__ __forceinline__ float dsilu_f(float z) {
@@ -30,24 +43,8 @@ __device__ __forceinline__ float dsilu_f(float z) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// C[M,N] = epilogue( op(A)[M,K] W[K,N] (+ A2[M,K2] W2[K2,N]) )
+// C[M,N] = epilogue( op(A)[M,K] W[K,N] (+ A2[M,K2] W2[K2,N]) )   (GemmArgs)
 // ------------------------------------------------------------------------------------------------
-struct GemmArgs {
-  const float* A;
-  const float* A2;
-  const float* W;
-  const float* W2;
-  const float* bias;    // [N]
-  const float* rowvec;  // [M / rows_per_vec, N]
-  int rows_per_vec;
-  const float* resid;   // [M,N], added
-  const float* add;     // [M,N], added before the multiplication
-  const float* mulz;    // [M,N], multiply by silu'(mulz)
-  float* C;
-  int M;
-  int a_op;  // 1: silu on A while loading
-};
-
 template <int K, int N>
 struct GemmGeo {
   static constexpr int TR = (K == 256 || N == 256) ? 64 : 128;
@@ -124,12 +121,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_rows_kernel(const __grid_con
 }
 
 template <int K, int N, int K2>
-int launch_gemm(const GemmArgs& g, int num_sms, cudaStream_t st) {
-  // the big square edge-row GEMMs go to the tensor cores (ecnf_train_tc.cuh) unless the SIMT engine is forced
-  if constexpr (K == N && (K == 128 || K == 256)) {
-    if (!g.A2 && g.M >= 8192 && t_engine == 0) {
-      ecnf_train_tc::Args a{g.A, g.W, g.bias, g.rowvec, g.rows_per_vec, g.resid, g.add, g.mulz, g.C, g.M, g.a_op};
-      ECNF_CHECK_CUDA((ecnf_train_tc::launch<K, N>(a, num_sms, st)));
+int launch_gemm(const LaunchCtx& lc, const GemmArgs& g) {
+  if constexpr (tc_shape(K, N)) {
+    if (use_tc(lc, K, N, g.M, !g.A2 && !g.rowvec)) {
+      ECNF_CHECK_CUDA((ecnf_train_tc::launch<K, N>(g, lc.num_sms, lc.st)));
       return ECNF_OK;
     }
   }
@@ -142,8 +137,8 @@ int launch_gemm(const GemmArgs& g, int num_sms, cudaStream_t st) {
     configured = true;
   }
   const int ntiles = (g.M + TR - 1) / TR;
-  const int grid = std::min(ntiles, num_sms * 8);
-  kern<<<grid, NTHREADS, smem, st>>>(g);
+  const int grid = std::min(ntiles, lc.num_sms * 8);
+  kern<<<grid, NTHREADS, smem, lc.st>>>(g);
   ECNF_CHECK_CUDA(cudaGetLastError());
   return ECNF_OK;
 }
@@ -232,36 +227,35 @@ __global__ void __launch_bounds__(NTHREADS) dw_kernel(const float* __restrict__ 
 }
 
 __global__ void colsum_kernel(const float* __restrict__ Z, int M, int N, float* __restrict__ out, int rows_per_cta);
-// rows per CTA of colsum_kernel: >= 4 CTAs per SM for the big (edge-row) matrices, enough CTAs to cover the latency for the
-// node-row ones (9 728 rows in 38 CTAs took 27 us per launch)
-inline int colsum_rows(long long M) { return M >= 65536 ? 256 : 32; }
+// out[N] += column sums of Z[M,N].  Rows per CTA: >= 4 CTAs per SM for the big (edge-row) matrices, enough CTAs to cover
+// the latency for the node-row ones (9 728 rows in 38 CTAs took 27 us per launch)
+void launch_colsum(const LaunchCtx& lc, const float* Z, int M, int N, float* out) {
+  const int rows = M >= 65536 ? 256 : 32;
+  colsum_kernel<<<(unsigned)((M + rows - 1) / rows), NTHREADS, 0, lc.st>>>(Z, M, N, out, rows);
+}
 
 // dW += op(A)^T dZ; bias_grad (optional) += column sums of dZ (fused into the tensor-core kernel, else a second launch)
-int launch_dw(const float* A, int lda, int a_op, const float* dZ, int ldz, float* dW, int K, int N, int M, int num_sms,
-              cudaStream_t st, float* bias_grad = nullptr) {
-  // the big square weight gradients (reduction over the edge rows) go to the tensor cores (ecnf_train_tc.cuh)
-  if (lda == K && ldz == N && K == N && (K == 128 || K == 256) && M >= 8192 && t_engine == 0) {
-    if (K == 256) ECNF_CHECK_CUDA((ecnf_train_tc::launch_dw<256, 256>(A, a_op, dZ, dW, bias_grad, M, num_sms, st)));
-    else ECNF_CHECK_CUDA((ecnf_train_tc::launch_dw<128, 128>(A, a_op, dZ, dW, bias_grad, M, num_sms, st)));
+int launch_dw(const LaunchCtx& lc, const float* A, int lda, int a_op, const float* dZ, int ldz, float* dW, int K, int N,
+              int M, float* bias_grad = nullptr) {
+  if (use_tc(lc, K, N, M, lda == K && ldz == N)) {
+    if (K == 256) ECNF_CHECK_CUDA((ecnf_train_tc::launch_dw<256, 256>(A, a_op, dZ, dW, bias_grad, M, lc.num_sms, lc.st)));
+    else ECNF_CHECK_CUDA((ecnf_train_tc::launch_dw<128, 128>(A, a_op, dZ, dW, bias_grad, M, lc.num_sms, lc.st)));
     return ECNF_OK;
   }
-  if (bias_grad) {
-    const int rows = colsum_rows(M);
-    colsum_kernel<<<(unsigned)((M + rows - 1) / rows), NTHREADS, 0, st>>>(dZ, M, N, bias_grad, rows);
-  }
+  if (bias_grad) launch_colsum(lc, dZ, M, N, bias_grad);
   // block shape: 128 where the dimension allows, else 64 / 32
   auto pick = [](int d) { return d % 128 == 0 ? 128 : (d % 64 == 0 ? 64 : 32); };
   const int BK = pick(K), BN = pick(N);
   const int nb = (K / BK) * (N / BN);
-  int nslabs = std::max(1, (num_sms * 2) / nb);
+  int nslabs = std::max(1, (lc.num_sms * 2) / nb);
   int rows_per_cta = ((M + nslabs - 1) / nslabs + 31) / 32 * 32;
   nslabs = (M + rows_per_cta - 1) / rows_per_cta;
   dim3 grid(nslabs, K / BK, N / BN);
-#define DW_CASE(bk, bn)                                                                        \
-  if (BK == bk && BN == bn) {                                                                  \
-    dw_kernel<bk, bn><<<grid, NTHREADS, 0, st>>>(A, lda, a_op, dZ, ldz, dW, N, M, rows_per_cta); \
-    ECNF_CHECK_CUDA(cudaGetLastError());                                                       \
-    return ECNF_OK;                                                                            \
+#define DW_CASE(bk, bn)                                                                             \
+  if (BK == bk && BN == bn) {                                                                       \
+    dw_kernel<bk, bn><<<grid, NTHREADS, 0, lc.st>>>(A, lda, a_op, dZ, ldz, dW, N, M, rows_per_cta); \
+    ECNF_CHECK_CUDA(cudaGetLastError());                                                            \
+    return ECNF_OK;                                                                                 \
   }
   DW_CASE(128, 128) DW_CASE(128, 64) DW_CASE(64, 128) DW_CASE(64, 64) DW_CASE(32, 128) DW_CASE(128, 32) DW_CASE(32, 64)
   DW_CASE(64, 32) DW_CASE(32, 32)
@@ -768,64 +762,66 @@ __global__ void embed_bwd_kernel(Dims d, const int32_t* __restrict__ feat, const
 // ------------------------------------------------------------------------------------------------
 // host orchestration
 // ------------------------------------------------------------------------------------------------
-struct Arena {
-  char* base;
-  size_t off, cap;
-  float* take(size_t nfloats) {
-    size_t bytes = (nfloats * sizeof(float) + 255) & ~(size_t)255;
-    float* p = reinterpret_cast<float*>(base + off);
-    off += bytes;
-    return p;
-  }
+// Graphs per chunk of a minibatch (ecnf_model_set_fm_chunk; 0 = the whole minibatch in one pass); the gradients of the
+// chunks accumulate
+int64_t fm_chunk_graphs(const ecnf_model* m, int64_t B) { return m->fm_chunk > 0 && m->fm_chunk < B ? m->fm_chunk : B; }
+
+// Every buffer of the workspace of one chunk
+struct FmWorkspace {
+  float *ut, *mu, *tau, *xs[ECNF_MAX_BLOCKS + 1], *dxs[2], *cvec;
+  float *hprev[ECNF_MAX_BLOCKS + 1], *hin[ECNF_MAX_BLOCKS];
+  float *Ps, *Pr;   // also dPs, dPr
+  float *Mb[ECNF_MAX_BLOCKS], *Zh[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS];
+  float *Ze[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS], *Zx[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS];
+  float *pb[ECNF_MAX_BLOCKS], *eb[ECNF_MAX_BLOCKS];
+  float *DM, *dvgeo, *dM, *dhin, *dh[2];
+  float* Wt;   // transposed weights, at the offsets of the parameter layout
 };
 
-// Graphs per chunk of a minibatch (ecnf_model_set_fm_chunk; 0 = automatic).  A chunk's [edge rows x U] fp32 matrices are
-// sized to stay (mostly) resident in the 126 MB L2 between the kernel that writes one and the kernel that reads it, so the
-// layer-by-layer GEMMs read their operand from L2 instead of HBM; the gradients of the chunks accumulate.
-constexpr int64_t ECNF_FM_CHUNK_BYTES = 1LL << 40;   // automatic chunking: bytes of one [edge rows x U] fp32 matrix per chunk
-int64_t fm_chunk_graphs(const ecnf_model* m, int64_t B) {
-  int64_t c = m->fm_chunk;
-  if (c <= 0) {
-    const ecnf_config& cf = m->cfg;
-    const int64_t bytes_per_graph = (int64_t)cf.n_frames * (cf.n_frames - 1) * cf.mlp_units * 4;
-    c = ECNF_FM_CHUNK_BYTES / bytes_per_graph;
-    if (c < 1) c = 1;
-    const int64_t nchunks = (B + c - 1) / c;          // equal chunks
-    c = (B + nchunks - 1) / nchunks;
-  }
-  return c < B ? c : B;
-}
-
-size_t fm_bytes(const ecnf_model* m, int64_t B) {
+// Lays out the buffers of a chunk of `Bws` graphs from `base` into `w` (256-byte aligned) and returns the bytes they
+// take.  With a null base it only counts: ecnf_fm_workspace_bytes sizes the workspace with it.
+size_t fm_layout(const ecnf_model* m, int64_t Bws, void* base, FmWorkspace& w) {
   const ecnf_config& c = m->cfg;
-  const size_t n = c.n_frames, D = n * c.dim, E = n * (n - 1), H = c.n_hidden, U = c.mlp_units, T = c.time_dim,
-               L = c.n_layers, nb = c.n_blocks;
-  const size_t NB = B * n, EB = B * E;
-  auto r = [](size_t f) { return (f * 4 + 255) & ~(size_t)255; };
-  size_t s = 256;
-  s += r(8);                                            // freqs
-  s += r(B * D) + r(B * 4) + r(B * T);                  // ut, mu, tau
-  s += (nb + 1) * r(B * D);                             // xs[b]
-  s += 2 * r(B * D);                                    // dxs ping-pong
-  s += r(B * H);                                        // cvec
-  s += (nb + 1) * r(NB * H) + nb * r(NB * H);           // hprev[b] (+ output of last), hin[b]
-  s += 2 * r(NB * U);                                   // Ps, Pr (also dPs, dPr)
-  s += nb * r(NB * U);                                  // M[b]
-  s += nb * L * r(NB * U);                              // Zh[b][l]
-  s += 2 * nb * L * r(EB * U);                          // Ze, Zx
-  s += 2 * nb * r(EB);                                  // p, eatt
-  s += r(EB * U) + r(EB * 4);                           // DM, dvgeo
-  s += r(NB * U) + 3 * r(NB * H);                       // dM, dhin, dh x2
-  s += r((size_t)m->param_count);                       // transposed weights
-  return s;
+  const size_t n = c.n_frames, D = n * c.dim, H = c.n_hidden, U = c.mlp_units, T = c.time_dim;
+  const size_t B = (size_t)Bws, NB = B * n, EB = B * n * (n - 1);
+  const int nb = c.n_blocks, L = c.n_layers;
+  size_t off = 256;
+  auto take = [&](size_t nfloats) {
+    float* p = base ? reinterpret_cast<float*>(static_cast<char*>(base) + off) : nullptr;
+    off += (nfloats * sizeof(float) + 255) & ~(size_t)255;
+    return p;
+  };
+  w.ut = take(B * D);
+  w.mu = take(B * 4);
+  w.tau = take(B * T);
+  for (int b = 0; b <= nb; ++b) w.xs[b] = take(B * D);
+  for (float*& p : w.dxs) p = take(B * D);
+  w.cvec = take(B * H);
+  for (int b = 0; b <= nb; ++b) w.hprev[b] = take(NB * H);
+  for (int b = 0; b < nb; ++b) w.hin[b] = take(NB * H);
+  w.Ps = take(NB * U);
+  w.Pr = take(NB * U);
+  for (int b = 0; b < nb; ++b) w.Mb[b] = take(NB * U);
+  for (int b = 0; b < nb; ++b)
+    for (int l = 0; l < L; ++l) w.Zh[b][l] = take(NB * U);
+  for (int b = 0; b < nb; ++b)
+    for (int l = 0; l < L; ++l) { w.Ze[b][l] = take(EB * U); w.Zx[b][l] = take(EB * U); }
+  for (int b = 0; b < nb; ++b) { w.pb[b] = take(EB); w.eb[b] = take(EB); }
+  w.DM = take(EB * U);
+  w.dvgeo = take(EB * 4);
+  w.dM = take(NB * U);
+  w.dhin = take(NB * H);
+  for (float*& p : w.dh) p = take(NB * H);
+  w.Wt = take((size_t)m->param_count);
+  return off;
 }
 
-// One chunk of `B` graphs (rows [0, B) of the pointers given) through forward + backward.  The workspace is carved for
+// One chunk of `B` graphs (rows [0, B) of the pointers given) through forward + backward.  The workspace is laid out for
 // `Bws` >= B graphs; every gradient (and the loss) is ACCUMULATED, so the chunks of a minibatch add up.  `first`: clear the
 // gradient / loss and transpose the weights (once per minibatch).
 template <int U, int H>
 int fm_run(const ecnf_model* m, const float* x_data, const float* x0, const float* t, const int32_t* feat, int64_t B,
-           int64_t Bws, bool first, float denom, float* out_loss, float* out_grad, void* ws, cudaStream_t st) {
+           int64_t Bws, bool first, float denom, float* out_loss, float* out_grad, void* ws, const LaunchCtx& lc) {
   const ecnf_config& c = m->cfg;
   const EcnfModelDev md = ecnf_make_dev(m, m->d_params);
   const EcnfModelDev gd = ecnf_make_dev(m, out_grad);  // same layout, pointing into the gradient buffer
@@ -833,43 +829,12 @@ int fm_run(const ecnf_model* m, const float* x_data, const float* x0, const floa
   d.B = (int)B; d.n = c.n_frames; d.dim = c.dim; d.D = d.n * d.dim; d.E = d.n * (d.n - 1); d.H = H; d.U = U;
   d.T = c.time_dim; d.L = c.n_layers; d.nfeat = c.n_features; d.C = c.normalization_constant; d.sigma_min = c.sigma_min;
   for (int k = 0; k < 8; ++k) d.freqs[k] = c.freqs[k];
-  const int nb = c.n_blocks, L = c.n_layers, sms = m->num_sms;
+  const int nb = c.n_blocks, L = c.n_layers;
   const size_t NB = (size_t)B * d.n, EB = (size_t)B * d.E;
-  const size_t Bw = (size_t)Bws, NBw = Bw * d.n, EBw = Bw * d.E;   // carve-up sizes (the same for every chunk)
-  Arena ar{reinterpret_cast<char*>(ws), 256, 0};
-  ar.take(8);   // (was: a device copy of the frequency table)
-  float* ut = ar.take(Bw * d.D);
-  float* mu = ar.take(Bw * 4);
-  float* tau = ar.take(Bw * d.T);
-  float* xs[ECNF_MAX_BLOCKS + 1];
-  for (int b = 0; b <= nb; ++b) xs[b] = ar.take(Bw * d.D);
-  float* dxs[2] = {ar.take(Bw * d.D), ar.take(Bw * d.D)};
-  float* cvec = ar.take(Bw * H);
-  float* hprev[ECNF_MAX_BLOCKS + 1];
-  float* hin[ECNF_MAX_BLOCKS];
-  for (int b = 0; b <= nb; ++b) hprev[b] = ar.take(NBw * H);
-  for (int b = 0; b < nb; ++b) hin[b] = ar.take(NBw * H);
-  float* Ps = ar.take(NBw * U);
-  float* Pr = ar.take(NBw * U);
-  float* Mb[ECNF_MAX_BLOCKS];
-  float* Zh[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS];
-  float* Ze[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS];
-  float* Zx[ECNF_MAX_BLOCKS][ECNF_MAX_LAYERS];
-  float* pb[ECNF_MAX_BLOCKS];
-  float* eb[ECNF_MAX_BLOCKS];
-  for (int b = 0; b < nb; ++b) Mb[b] = ar.take(NBw * U);
-  for (int b = 0; b < nb; ++b)
-    for (int l = 0; l < L; ++l) Zh[b][l] = ar.take(NBw * U);
-  for (int b = 0; b < nb; ++b)
-    for (int l = 0; l < L; ++l) { Ze[b][l] = ar.take(EBw * U); Zx[b][l] = ar.take(EBw * U); }
-  for (int b = 0; b < nb; ++b) { pb[b] = ar.take(EBw); eb[b] = ar.take(EBw); }
-  float* DM = ar.take(EBw * U);
-  float* dvgeo = ar.take(EBw * 4);
-  float* dM = ar.take(NBw * U);
-  float* dhin = ar.take(NBw * H);
-  float* dh[2] = {ar.take(NBw * H), ar.take(NBw * H)};
-  float* Wt = ar.take((size_t)m->param_count);
-  const EcnfModelDev td = ecnf_make_dev(m, Wt);  // transposed weights live at the same offsets
+  const cudaStream_t st = lc.st;
+  FmWorkspace w;
+  fm_layout(m, Bws, ws, w);
+  const EcnfModelDev td = ecnf_make_dev(m, w.Wt);  // transposed weights live at the same offsets
 
   if (first) {
     ECNF_CHECK_CUDA(cudaMemsetAsync(out_grad, 0, (size_t)m->param_count * sizeof(float), st));
@@ -914,143 +879,139 @@ int fm_run(const ecnf_model* m, const float* x_data, const float* x0, const floa
   int rc;
 
   // ------------------------------ forward ------------------------------
-  fm_prep_kernel<<<(unsigned)B, 128, 0, st>>>(d, x_data, x0, t, feat, md.embed, ut, mu, xs[0], tau, hprev[0]);
+  fm_prep_kernel<<<(unsigned)B, 128, 0, st>>>(d, x_data, x0, t, feat, md.embed, w.ut, w.mu, w.xs[0], w.tau, w.hprev[0]);
   for (int b = 0; b < nb; ++b) {
     const EcnfBlockParams& p = md.blk[b];
     const bool last = (b == nb - 1);
-    tau_proj_kernel<<<(unsigned)((B * H + 255) / 256), 256, 0, st>>>(d, tau, p.Wd, p.bd, cvec);
+    tau_proj_kernel<<<(unsigned)((B * H + 255) / 256), 256, 0, st>>>(d, w.tau, p.Wd, p.bd, w.cvec);
     {
-      GemmArgs g = gemm_args(hprev[b], p.Wd, hin[b], (int)NB);
-      g.rowvec = cvec; g.rows_per_vec = d.n;
-      if ((rc = launch_gemm<H, H, 0>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.hprev[b], p.Wd, w.hin[b], (int)NB);
+      g.rowvec = w.cvec; g.rows_per_vec = d.n;
+      if ((rc = launch_gemm<H, H, 0>(lc, g))) return rc;
     }
     {
-      GemmArgs g = gemm_args(hin[b], p.We[0], Ps, (int)NB);
-      if ((rc = launch_gemm<H, U, 0>(g, sms, st))) return rc;
-      g = gemm_args(hin[b], p.We[0] + (size_t)H * U, Pr, (int)NB);
+      GemmArgs g = gemm_args(w.hin[b], p.We[0], w.Ps, (int)NB);
+      if ((rc = launch_gemm<H, U, 0>(lc, g))) return rc;
+      g = gemm_args(w.hin[b], p.We[0] + (size_t)H * U, w.Pr, (int)NB);
       g.bias = p.be[0];
-      if ((rc = launch_gemm<H, U, 0>(g, sms, st))) return rc;
+      if ((rc = launch_gemm<H, U, 0>(lc, g))) return rc;
     }
     edge_gather_kernel<<<(unsigned)((EB * (U / 4) + ew_threads - 1) / ew_threads), ew_threads, 0, st>>>(
-        d, xs[b], Ps, Pr, p.We[0] + (size_t)2 * H * U, Ze[b][0]);
+        d, w.xs[b], w.Ps, w.Pr, p.We[0] + (size_t)2 * H * U, w.Ze[b][0]);
     for (int l = 1; l < L; ++l) {
-      GemmArgs g = gemm_args(Ze[b][l - 1], p.We[l], Ze[b][l], (int)EB);
+      GemmArgs g = gemm_args(w.Ze[b][l - 1], p.We[l], w.Ze[b][l], (int)EB);
       g.a_op = 1; g.bias = p.be[l];
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
     }
     for (int l = 0; l < L; ++l) {
-      GemmArgs g = gemm_args(l == 0 ? Ze[b][L - 1] : Zx[b][l - 1], p.Wx[l], Zx[b][l], (int)EB);
+      GemmArgs g = gemm_args(l == 0 ? w.Ze[b][L - 1] : w.Zx[b][l - 1], p.Wx[l], w.Zx[b][l], (int)EB);
       g.a_op = 1; g.bias = p.bx[l];
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
     }
-    edge_heads_kernel<U><<<(unsigned)((EB + 7) / 8), 256, 0, st>>>(d, Ze[b][L - 1], Zx[b][L - 1], p.wa, p.ba, p.wp, p.bp,
-                                                                 eb[b], pb[b]);
-    node_aggregate_kernel<<<(unsigned)NB, U / 4 < 32 ? 32 : U / 4, 0, st>>>(d, xs[b], Ze[b][L - 1], eb[b], pb[b], Mb[b], xs[b + 1], !last);
+    edge_heads_kernel<U><<<(unsigned)((EB + 7) / 8), 256, 0, st>>>(d, w.Ze[b][L - 1], w.Zx[b][L - 1], p.wa, p.ba, p.wp, p.bp,
+                                                                 w.eb[b], w.pb[b]);
+    node_aggregate_kernel<<<(unsigned)NB, U / 4 < 32 ? 32 : U / 4, 0, st>>>(d, w.xs[b], w.Ze[b][L - 1], w.eb[b], w.pb[b], w.Mb[b], w.xs[b + 1], !last);
     if (!last) {
-      GemmArgs g = gemm_args(Mb[b], p.Wh[0], Zh[b][0], (int)NB);
-      g.A2 = hin[b]; g.W2 = p.Wh[0] + (size_t)U * U; g.bias = p.bh[0];
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.Mb[b], p.Wh[0], w.Zh[b][0], (int)NB);
+      g.A2 = w.hin[b]; g.W2 = p.Wh[0] + (size_t)U * U; g.bias = p.bh[0];
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
       for (int l = 1; l < L; ++l) {
-        g = gemm_args(Zh[b][l - 1], p.Wh[l], Zh[b][l], (int)NB);
+        g = gemm_args(w.Zh[b][l - 1], p.Wh[l], w.Zh[b][l], (int)NB);
         g.a_op = 1; g.bias = p.bh[l];
-        if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+        if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
       }
-      g = gemm_args(Zh[b][L - 1], p.Wh[L], hprev[b + 1], (int)NB);
-      g.a_op = 1; g.bias = p.bh[L]; g.resid = hin[b];
-      if ((rc = launch_gemm<U, H, 0>(g, sms, st))) return rc;
+      g = gemm_args(w.Zh[b][L - 1], p.Wh[L], w.hprev[b + 1], (int)NB);
+      g.a_op = 1; g.bias = p.bh[L]; g.resid = w.hin[b];
+      if ((rc = launch_gemm<U, H, 0>(lc, g))) return rc;
     }
   }
-  loss_kernel<<<(unsigned)((B * d.D + 255) / 256), 256, 0, st>>>(d, xs[nb], xs[0], mu, ut, md.final_scaling, denom, out_loss,
-                                                               dxs[0], const_cast<float*>(gd.final_scaling));
+  loss_kernel<<<(unsigned)((B * d.D + 255) / 256), 256, 0, st>>>(d, w.xs[nb], w.xs[0], w.mu, w.ut, md.final_scaling, denom, out_loss,
+                                                               w.dxs[0], const_cast<float*>(gd.final_scaling));
   ECNF_CHECK_CUDA(cudaGetLastError());
 
   // ------------------------------ backward ------------------------------
   int cur = 0;        // dxs[cur] = grad wrt coordinates leaving block b
   int hcur = 0;       // dh[hcur] = grad wrt h leaving block b (valid for b < nb-1)
-  auto colsum = [&](const float* Z, size_t M, int N, const float* out) {
-    const int rows = colsum_rows((long long)M);
-    colsum_kernel<<<(unsigned)((M + rows - 1) / rows), NTHREADS, 0, st>>>(Z, (int)M, N, const_cast<float*>(out), rows);
-  };
   for (int b = nb - 1; b >= 0; --b) {
     const EcnfBlockParams &p = md.blk[b], &q = td.blk[b], &gp = gd.blk[b];
     const bool last = (b == nb - 1);
     bool dhin_valid = false;
     if (!last) {
       // h_out = phi_h([M | h_in]) + h_in
-      const float* dho = dh[hcur];
-      if ((rc = launch_dw(Zh[b][L - 1], U, 1, dho, H, const_cast<float*>(gp.Wh[L]), U, H, (int)NB, sms, st))) return rc;
-      colsum(dho, NB, H, gp.bh[L]);
-      GemmArgs g = gemm_args(dho, q.Wh[L], Zh[b][L - 1], (int)NB);   // [NB,H] x [H,U]
-      g.mulz = Zh[b][L - 1];
-      if ((rc = launch_gemm<H, U, 0>(g, sms, st))) return rc;
+      const float* dho = w.dh[hcur];
+      if ((rc = launch_dw(lc, w.Zh[b][L - 1], U, 1, dho, H, const_cast<float*>(gp.Wh[L]), U, H, (int)NB))) return rc;
+      launch_colsum(lc, dho, (int)NB, H, const_cast<float*>(gp.bh[L]));
+      GemmArgs g = gemm_args(dho, q.Wh[L], w.Zh[b][L - 1], (int)NB);   // [NB,H] x [H,U]
+      g.mulz = w.Zh[b][L - 1];
+      if ((rc = launch_gemm<H, U, 0>(lc, g))) return rc;
       for (int l = L - 1; l >= 1; --l) {
-        if ((rc = launch_dw(Zh[b][l - 1], U, 1, Zh[b][l], U, const_cast<float*>(gp.Wh[l]), U, U, (int)NB, sms, st))) return rc;
-        colsum(Zh[b][l], NB, U, gp.bh[l]);
-        g = gemm_args(Zh[b][l], q.Wh[l], Zh[b][l - 1], (int)NB);
-        g.mulz = Zh[b][l - 1];
-        if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+        if ((rc = launch_dw(lc, w.Zh[b][l - 1], U, 1, w.Zh[b][l], U, const_cast<float*>(gp.Wh[l]), U, U, (int)NB))) return rc;
+        launch_colsum(lc, w.Zh[b][l], (int)NB, U, const_cast<float*>(gp.bh[l]));
+        g = gemm_args(w.Zh[b][l], q.Wh[l], w.Zh[b][l - 1], (int)NB);
+        g.mulz = w.Zh[b][l - 1];
+        if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
       }
-      if ((rc = launch_dw(Mb[b], U, 0, Zh[b][0], U, const_cast<float*>(gp.Wh[0]), U, U, (int)NB, sms, st))) return rc;
-      if ((rc = launch_dw(hin[b], H, 0, Zh[b][0], U, const_cast<float*>(gp.Wh[0]) + (size_t)U * U, H, U, (int)NB, sms, st))) return rc;
-      colsum(Zh[b][0], NB, U, gp.bh[0]);
-      g = gemm_args(Zh[b][0], q.Wh[0], dM, (int)NB);
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
-      g = gemm_args(Zh[b][0], q.Wh[0] + (size_t)U * U, dhin, (int)NB);   // [NB,U] x [U,H]
+      if ((rc = launch_dw(lc, w.Mb[b], U, 0, w.Zh[b][0], U, const_cast<float*>(gp.Wh[0]), U, U, (int)NB))) return rc;
+      if ((rc = launch_dw(lc, w.hin[b], H, 0, w.Zh[b][0], U, const_cast<float*>(gp.Wh[0]) + (size_t)U * U, H, U, (int)NB))) return rc;
+      launch_colsum(lc, w.Zh[b][0], (int)NB, U, const_cast<float*>(gp.bh[0]));
+      g = gemm_args(w.Zh[b][0], q.Wh[0], w.dM, (int)NB);
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
+      g = gemm_args(w.Zh[b][0], q.Wh[0] + (size_t)U * U, w.dhin, (int)NB);   // [NB,U] x [U,H]
       g.resid = dho;
-      if ((rc = launch_gemm<U, H, 0>(g, sms, st))) return rc;
+      if ((rc = launch_gemm<U, H, 0>(lc, g))) return rc;
       dhin_valid = true;
     }
     // attention / head / coordinate update
-    heads_bwd_kernel<U><<<heads_grid, 256, 0, st>>>(d, xs[b], Ze[b][L - 1], Zx[b][L - 1], eb[b], pb[b], last ? nullptr : dM,
-                                                   dxs[cur], p.wa, p.wp, DM, dvgeo, const_cast<float*>(gp.wa),
+    heads_bwd_kernel<U><<<heads_grid, 256, 0, st>>>(d, w.xs[b], w.Ze[b][L - 1], w.Zx[b][L - 1], w.eb[b], w.pb[b], last ? nullptr : w.dM,
+                                                   w.dxs[cur], p.wa, p.wp, w.DM, w.dvgeo, const_cast<float*>(gp.wa),
                                                    const_cast<float*>(gp.ba), const_cast<float*>(gp.wp),
                                                    const_cast<float*>(gp.bp), rows_per_warp);
     // phi_x chain
     for (int l = L - 1; l >= 0; --l) {
-      const float* Ain = (l == 0) ? Ze[b][L - 1] : Zx[b][l - 1];
-      if ((rc = launch_dw(Ain, U, 1, Zx[b][l], U, const_cast<float*>(gp.Wx[l]), U, U, (int)EB, sms, st,
+      const float* Ain = (l == 0) ? w.Ze[b][L - 1] : w.Zx[b][l - 1];
+      if ((rc = launch_dw(lc, Ain, U, 1, w.Zx[b][l], U, const_cast<float*>(gp.Wx[l]), U, U, (int)EB,
                           const_cast<float*>(gp.bx[l])))) return rc;
-      GemmArgs g = gemm_args(Zx[b][l], q.Wx[l], l == 0 ? Ze[b][L - 1] : Zx[b][l - 1], (int)EB);
-      g.mulz = (l == 0) ? Ze[b][L - 1] : Zx[b][l - 1];
-      if (l == 0) g.add = DM;
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.Zx[b][l], q.Wx[l], l == 0 ? w.Ze[b][L - 1] : w.Zx[b][l - 1], (int)EB);
+      g.mulz = (l == 0) ? w.Ze[b][L - 1] : w.Zx[b][l - 1];
+      if (l == 0) g.add = w.DM;
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
     }
     // phi_e chain
     for (int l = L - 1; l >= 1; --l) {
-      if ((rc = launch_dw(Ze[b][l - 1], U, 1, Ze[b][l], U, const_cast<float*>(gp.We[l]), U, U, (int)EB, sms, st,
+      if ((rc = launch_dw(lc, w.Ze[b][l - 1], U, 1, w.Ze[b][l], U, const_cast<float*>(gp.We[l]), U, U, (int)EB,
                           const_cast<float*>(gp.be[l])))) return rc;
-      GemmArgs g = gemm_args(Ze[b][l], q.We[l], Ze[b][l - 1], (int)EB);
-      g.mulz = Ze[b][l - 1];
-      if ((rc = launch_gemm<U, U, H>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.Ze[b][l], q.We[l], w.Ze[b][l - 1], (int)EB);
+      g.mulz = w.Ze[b][l - 1];
+      if ((rc = launch_gemm<U, U, H>(lc, g))) return rc;
     }
     // first phi_e layer: gather backward
     // first phi_e layer: d|v|^2 -> dvgeo, d w_d and the bias gradient (column sums of dZ_e0) in one pass over dZ_e0
-    gather_bwd_edge_kernel<U><<<heads_grid, 256, 0, st>>>(d, xs[b], Ze[b][0], p.We[0] + (size_t)2 * H * U, dvgeo,
+    gather_bwd_edge_kernel<U><<<heads_grid, 256, 0, st>>>(d, w.xs[b], w.Ze[b][0], p.We[0] + (size_t)2 * H * U, w.dvgeo,
                                                          const_cast<float*>(gp.We[0]) + (size_t)2 * H * U,
                                                          const_cast<float*>(gp.be[0]), rows_per_warp);
-    gather_bwd_node_kernel<<<(unsigned)NB, U / 4 < 32 ? 32 : U / 4, 0, st>>>(d, Ze[b][0], dvgeo, dxs[cur], Ps, Pr, b > 0 ? dxs[cur ^ 1] : nullptr);
-    if ((rc = launch_dw(hin[b], H, 0, Ps, U, const_cast<float*>(gp.We[0]), H, U, (int)NB, sms, st))) return rc;
-    if ((rc = launch_dw(hin[b], H, 0, Pr, U, const_cast<float*>(gp.We[0]) + (size_t)H * U, H, U, (int)NB, sms, st))) return rc;
+    gather_bwd_node_kernel<<<(unsigned)NB, U / 4 < 32 ? 32 : U / 4, 0, st>>>(d, w.Ze[b][0], w.dvgeo, w.dxs[cur], w.Ps, w.Pr, b > 0 ? w.dxs[cur ^ 1] : nullptr);
+    if ((rc = launch_dw(lc, w.hin[b], H, 0, w.Ps, U, const_cast<float*>(gp.We[0]), H, U, (int)NB))) return rc;
+    if ((rc = launch_dw(lc, w.hin[b], H, 0, w.Pr, U, const_cast<float*>(gp.We[0]) + (size_t)H * U, H, U, (int)NB))) return rc;
     {
-      GemmArgs g = gemm_args(Ps, q.We[0], dhin, (int)NB);   // [NB,U] x [U,H]
-      if (dhin_valid) g.resid = dhin;
-      if ((rc = launch_gemm<U, H, 0>(g, sms, st))) return rc;
-      g = gemm_args(Pr, q.We[0] + (size_t)H * U, dhin, (int)NB);
-      g.resid = dhin;
-      if ((rc = launch_gemm<U, H, 0>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.Ps, q.We[0], w.dhin, (int)NB);   // [NB,U] x [U,H]
+      if (dhin_valid) g.resid = w.dhin;
+      if ((rc = launch_gemm<U, H, 0>(lc, g))) return rc;
+      g = gemm_args(w.Pr, q.We[0] + (size_t)H * U, w.dhin, (int)NB);
+      g.resid = w.dhin;
+      if ((rc = launch_gemm<U, H, 0>(lc, g))) return rc;
     }
     // h_in = [h | tau] Wd + bd
-    if ((rc = launch_dw(hprev[b], H, 0, dhin, H, const_cast<float*>(gp.Wd), H, H, (int)NB, sms, st))) return rc;
-    colsum(dhin, NB, H, gp.bd);
-    tau_grad_kernel<<<(unsigned)((B + 15) / 16), H * d.T, 0, st>>>(d, tau, dhin, const_cast<float*>(gp.Wd) + (size_t)H * H, 16);
+    if ((rc = launch_dw(lc, w.hprev[b], H, 0, w.dhin, H, const_cast<float*>(gp.Wd), H, H, (int)NB))) return rc;
+    launch_colsum(lc, w.dhin, (int)NB, H, const_cast<float*>(gp.bd));
+    tau_grad_kernel<<<(unsigned)((B + 15) / 16), H * d.T, 0, st>>>(d, w.tau, w.dhin, const_cast<float*>(gp.Wd) + (size_t)H * H, 16);
     {
-      GemmArgs g = gemm_args(dhin, q.Wd, dh[hcur ^ 1], (int)NB);
-      if ((rc = launch_gemm<H, H, 0>(g, sms, st))) return rc;
+      GemmArgs g = gemm_args(w.dhin, q.Wd, w.dh[hcur ^ 1], (int)NB);
+      if ((rc = launch_gemm<H, H, 0>(lc, g))) return rc;
       hcur ^= 1;
     }
     cur ^= 1;
   }
-  embed_bwd_kernel<<<(unsigned)((NB * H + 255) / 256), 256, 0, st>>>(d, feat, dh[hcur], const_cast<float*>(gd.embed));
+  embed_bwd_kernel<<<(unsigned)((NB * H + 255) / 256), 256, 0, st>>>(d, feat, w.dh[hcur], const_cast<float*>(gd.embed));
   ECNF_CHECK_CUDA(cudaGetLastError());
   return ECNF_OK;
 }
@@ -1061,7 +1022,8 @@ extern "C" {
 
 int64_t ecnf_fm_workspace_bytes(const ecnf_model* m, int64_t B) {
   if (!m || B <= 0) return 256;
-  return (int64_t)fm_bytes(m, fm_chunk_graphs(m, B));
+  FmWorkspace w;
+  return (int64_t)fm_layout(m, fm_chunk_graphs(m, B), nullptr, w);
 }
 
 int ecnf_fm_loss_grad(const ecnf_model* m, const float* x_data, const float* x0, const float* t, const int32_t* feat,
@@ -1080,8 +1042,7 @@ int ecnf_fm_loss_grad(const ecnf_model* m, const float* x_data, const float* x0,
     ecnf_set_error("workspace too small: need %lld bytes, got %lld", (long long)need, (long long)ws_bytes);
     return ECNF_ERR_WORKSPACE;
   }
-  cudaStream_t st = (cudaStream_t)stream;
-  t_engine = m->engine;
+  const LaunchCtx lc{m->num_sms, m->engine == 0, (cudaStream_t)stream};
   const int U = m->cfg.mlp_units, H = m->cfg.n_hidden;
   if (!((U == 128 && H == 64) || (U == 256 && H == 32) || (U == 64 && H == 32))) {
     ecnf_set_error("unsupported (mlp_units=%d, n_hidden=%d): compiled pairs are (128,64), (256,32), (64,32)", U, H);
@@ -1093,9 +1054,9 @@ int ecnf_fm_loss_grad(const ecnf_model* m, const float* x_data, const float* x0,
     const float *xd = x_data + b0 * D, *xz = x0 + b0 * D, *tt = t + b0;
     const int32_t* ft = feat + b0 * n;
     int rc;
-    if (U == 128) rc = fm_run<128, 64>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, st);
-    else if (U == 256) rc = fm_run<256, 32>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, st);
-    else rc = fm_run<64, 32>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, st);
+    if (U == 128) rc = fm_run<128, 64>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, lc);
+    else if (U == 256) rc = fm_run<256, 32>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, lc);
+    else rc = fm_run<64, 32>(m, xd, xz, tt, ft, bn, Bc, b0 == 0, loss_denominator, out_loss, out_grad, ws, lc);
     if (rc != ECNF_OK) return rc;
   }
   return ECNF_OK;

@@ -1,16 +1,13 @@
-// Engine B on the tensor cores: the big row-major GEMMs of the flow-matching step
-//     C[M, N] = epilogue( op(A)[M, K] x W[K, N] ),   M = B*n*(n-1) edge rows (175 k for QM9 at batch 512), K = N = mlp_units
-// (forward Dense layers and, with the pre-transposed weights, the backward-data GEMMs dA = dZ W^T) as tcgen05.mma with
-// the same 3-pass bf16 split as engine A (hi*hi + lo*hi + hi*lo, fp32 accumulate in TMEM, ~4e-6 relative error).
+// Engine B on the tensor cores: the GEMMs over the edge rows of the flow-matching step, M = B*n*(n-1) rows (175 k for
+// QM9 at batch 512), K = N = mlp_units = 128 or 256, as tcgen05.mma with the same 3-pass bf16 split as engine A
+// (hi*hi + lo*hi + hi*lo, fp32 accumulate in TMEM, ~4e-6 relative error):
 //
-//   * one persistent CTA per SM; a 128-row tile = the 128 TMEM lanes, thread (row, kh) owns row `row`;
-//   * A: coalesced loads (64 columns at a time) -> op (identity / SiLU) -> shared-memory stage -> the row's owner splits
-//     it to bf16 (hi, lo) and writes it into TENSOR MEMORY as the A operand (lane = row, one column = two consecutive k);
-//   * W: one 128-column half at a time, converted once per CTA into shared memory in the no-swizzle K-major canonical
-//     layout (the B operand); the row tiles then stream past it.  The CTAs of the two halves walk the tiles together, so
-//     A comes from HBM once (second read from L2);
-//   * epilogue: accumulator rows -> shared-memory stage -> coalesced pass (one warp = 512 contiguous bytes of a row):
-//     + bias, + per-graph row vector, + residual, + add, x silu'(z), fp32 store.
+//   * gemm_rows_tcT_kernel: C[M, N] = epilogue( op(A)[M, K] x W[K, N] ), the forward Dense layers and, with the
+//     pre-transposed weights, the backward-data GEMMs dA = dZ W^T; epilogue + bias, + residual, + add, x silu'(z);
+//   * dw_tc_kernel: dW[K, N] += op(A)[M, K]^T dZ[M, N], the weight gradients, with the bias gradient (the column sums of
+//     dZ) accumulated on the way.
+//
+// The launchers in ecnf_train.cu send a GEMM here only for these shapes; everything else runs on their fp32 SIMT kernels.
 #pragma once
 #include "ecnf_tc.cuh"
 
@@ -18,18 +15,22 @@ namespace ecnf_train_tc {
 
 using namespace ecnf_tc;
 
-struct Args {
+// One row GEMM  C[M, N] = epilogue( op(A)[M, K] W[K, N] (+ A2[M, K2] W2[K2, N]) ), for the SIMT kernel of ecnf_train.cu
+// and for gemm_rows_tcT_kernel, which supports neither A2 nor rowvec (the caller keeps such GEMMs on the SIMT kernel).
+struct GemmArgs {
   const float* A;
+  const float* A2;
   const float* W;
-  const float* bias;
-  const float* rowvec;
+  const float* W2;
+  const float* bias;    // [N]
+  const float* rowvec;  // [M / rows_per_vec, N]
   int rows_per_vec;
-  const float* resid;
-  const float* add;
-  const float* mulz;
+  const float* resid;   // [M,N], added
+  const float* add;     // [M,N], added before the multiplication
+  const float* mulz;    // [M,N], multiply by silu'(mulz)
   float* C;
   int M;
-  int a_op;
+  int a_op;  // 1: silu on A while loading
 };
 
 // ex2 / rcp based sigmoid (~1e-6 relative, well inside the 3-pass GEMM error): these elementwise ops run on 45 M elements
@@ -46,172 +47,8 @@ __device__ __forceinline__ float dsilu(float z) {
   return s * (1.f + z * (1.f - s));
 }
 
-constexpr int GEMM_NT = 512;    // 16 warps: thread (row, kq) = TMEM lane `row`, quarter kq of the columns it touches
-constexpr int STAGE_LD = 132;   // floats per staged row: 16-byte aligned, rows 8 apart share banks => float4 accesses by
-                                // 32 rows take the minimal 4 wavefronts
-
-template <int K, int N>
-__global__ void __launch_bounds__(GEMM_NT, 1) gemm_rows_tc_kernel(const __grid_constant__ Args g) {
-  static_assert((K == 128 || K == 256) && (N == 128 || N == 256), "shapes");
-  extern __shared__ __align__(1024) unsigned char smem[];
-  __nv_bfloat16* Whi = reinterpret_cast<__nv_bfloat16*>(smem);            // [128 n][K] canonical K-major
-  __nv_bfloat16* Wlo = Whi + 128 * K;
-  float* stage = reinterpret_cast<float*>(smem + (size_t)4 * 128 * K);    // [128 rows][STAGE_LD]: A chunks in, C tile out
-  __shared__ uint32_t tmem_slot;
-  __shared__ __align__(8) uint64_t mbar;
-  const int tid = threadIdx.x, warp = tid >> 5, row = tid & 127, kq = tid >> 7;
-  if (warp == 0) tmem_alloc(&tmem_slot, 512);
-  if (tid == 0) mbar_init(&mbar, 1);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = tmem_slot;
-  const uint32_t lane_addr = (uint32_t)(32 * (warp & 3)) << 16;
-  const uint32_t a_hi = tmem, a_lo = tmem + K / 2, acc0 = tmem + K;      // A: K columns, two accumulators of 128 columns
-  const int ntiles = (g.M + 127) / 128;
-
-  // CTA c works on column half (c % NH) of the row tiles c / NH, c / NH + grid / NH, ...: the CTAs of a group read the same
-  // A tiles at about the same time, so A comes from HBM once and from L2 for the other half
-  constexpr int NH = N / 128;
-  const int tile_step = gridDim.x / NH;
-  {
-    const int nh = blockIdx.x % NH;
-    // ---- W[:, 128 nh .. +128) -> bf16 hi / lo, canonical K-major with rows = n
-    for (int idx = tid; idx < K * 128; idx += GEMM_NT) {
-      const int k = idx >> 7, n = idx & 127;
-      const float w = g.W[(size_t)k * N + 128 * nh + n];
-      const __nv_bfloat16 h = __float2bfloat16(w);
-      const int d = canon_index(n, k, 128);
-      Whi[d] = h;
-      Wlo[d] = __float2bfloat16(w - __bfloat162float(h));
-    }
-    fence_proxy_async();
-    __syncthreads();
-    // A chunks (128 rows x 64 columns) are prefetched into registers one step ahead: the loads of chunk c+1 (or of the
-    // next tile's first chunk) are in flight while chunk c is converted / multiplied / written out
-    float4 nx[4];
-    auto fetch = [&](int tile_, int cb_) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int idx = tid + GEMM_NT * i, r = idx >> 4, c4 = idx & 15;
-        nx[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (tile_ < ntiles && tile_ * 128 + r < g.M)
-          nx[i] = *reinterpret_cast<const float4*>(g.A + (size_t)(tile_ * 128 + r) * K + cb_ * 64 + 4 * c4);
-      }
-    };
-    // epilogue of one tile: accumulator rows -> stage, then a coalesced pass (one warp = one 512-byte row segment)
-    auto epilogue = [&](int tile_, uint32_t acc_) {
-      const int r0 = tile_ * 128;
-      {
-        uint32_t x0[32];
-        tmem_ld32(acc_ + lane_addr + 32u * kq, x0);
-        tmem_wait_ld();
-        float* dst = stage + row * STAGE_LD + 32 * kq;
-#pragma unroll
-        for (int c4 = 0; c4 < 8; ++c4)
-          *reinterpret_cast<uint4*>(dst + 4 * c4) = make_uint4(x0[4 * c4], x0[4 * c4 + 1], x0[4 * c4 + 2], x0[4 * c4 + 3]);
-      }
-      tc_fence_before();
-      __syncthreads();
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const int idx = tid + GEMM_NT * i, r = idx >> 5, c4 = idx & 31;
-        if (r0 + r >= g.M) continue;
-        const size_t grow = (size_t)(r0 + r);
-        const int col = 128 * nh + 4 * c4;
-        float4 v = *reinterpret_cast<const float4*>(stage + r * STAGE_LD + 4 * c4);
-        if (g.bias) {
-          const float4 b = *reinterpret_cast<const float4*>(g.bias + col);
-          v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-        }
-        if (g.rowvec) {
-          const float4 b = *reinterpret_cast<const float4*>(g.rowvec + (grow / g.rows_per_vec) * N + col);
-          v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-        }
-        if (g.resid) {
-          const float4 b = *reinterpret_cast<const float4*>(g.resid + grow * N + col);
-          v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-        }
-        if (g.add) {
-          const float4 b = *reinterpret_cast<const float4*>(g.add + grow * N + col);
-          v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-        }
-        if (g.mulz) {
-          const float4 z = *reinterpret_cast<const float4*>(g.mulz + grow * N + col);
-          v.x *= dsilu(z.x); v.y *= dsilu(z.y); v.z *= dsilu(z.z); v.w *= dsilu(z.w);
-        }
-        *reinterpret_cast<float4*>(g.C + grow * N + col) = v;
-      }
-      __syncthreads();     // stage is rewritten by the next A chunk
-    };
-
-    // Pipeline: convert A(t) -> issue MMA(t) into accumulator t&1 -> epilogue of tile t-1 while MMA(t) runs.
-    fetch(blockIdx.x / NH, 0);
-    int prev_tile = -1;
-    uint32_t issued = 0;
-    for (int tile = blockIdx.x / NH; tile < ntiles; tile += tile_step) {
-      if (issued > 0) {      // the A operand in tensor memory is free once MMA(t-1) has completed
-        mbar_wait(&mbar, (issued - 1) & 1u);
-        tc_fence_after();
-      }
-#pragma unroll 1
-      for (int cb = 0; cb < K / 64; ++cb) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int idx = tid + GEMM_NT * i, r = idx >> 4, c4 = idx & 15;
-          float4 x = nx[i];
-          if (g.a_op) { x.x = silu(x.x); x.y = silu(x.y); x.z = silu(x.z); x.w = silu(x.w); }
-          *reinterpret_cast<float4*>(stage + r * STAGE_LD + 4 * c4) = x;
-        }
-        if (cb + 1 < K / 64) fetch(tile, cb + 1);
-        else fetch(tile + tile_step, 0);
-        __syncthreads();
-        uint32_t h[8], l[8];
-#pragma unroll
-        for (int c4 = 0; c4 < 4; ++c4) {
-          const float4 x = *reinterpret_cast<const float4*>(stage + row * STAGE_LD + 16 * kq + 4 * c4);
-          split_pack(x.x, x.y, h[2 * c4], l[2 * c4]);
-          split_pack(x.z, x.w, h[2 * c4 + 1], l[2 * c4 + 1]);
-        }
-        const uint32_t col = (uint32_t)(cb * 32 + kq * 8);
-        tmem_st8(a_hi + lane_addr + col, h);
-        tmem_st8(a_lo + lane_addr + col, l);
-        __syncthreads();     // stage is rewritten by the next chunk
-      }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncthreads();
-      if (tid == 0) {
-        tc_fence_after();
-        const uint32_t idesc = make_idesc_bf16(128, 128);
-        const uint32_t lbo = (128 / 8) * 128;
-        const uint32_t acc = acc0 + 128u * (issued & 1u);
-        for (int ks = 0; ks < K / 16; ++ks) {
-          const uint64_t bh = make_sdesc(smem_u32(Whi) + ks * 2 * lbo, lbo, 128);
-          const uint64_t bl = make_sdesc(smem_u32(Wlo) + ks * 2 * lbo, lbo, 128);
-          mma_ts(acc, a_hi + ks * 8, bh, idesc, ks > 0 ? 1u : 0u);
-          mma_ts(acc, a_lo + ks * 8, bh, idesc, 1u);
-          mma_ts(acc, a_hi + ks * 8, bl, idesc, 1u);
-        }
-        mma_commit(&mbar);
-      }
-      ++issued;
-      if (prev_tile >= 0) epilogue(prev_tile, acc0 + 128u * (issued & 1u));   // accumulator of MMA(t-1) = (issued - 2) & 1
-      prev_tile = tile;
-    }
-    if (prev_tile >= 0) {
-      mbar_wait(&mbar, (issued - 1) & 1u);
-      tc_fence_after();
-      epilogue(prev_tile, acc0 + 128u * ((issued - 1) & 1u));
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 512);
-}
-
 // =====================================================================================================================
-// Transposed, warp-specialised version of the same GEMM (the one the edge-row layers use):
+// C = epilogue( op(A) W ), transposed and warp-specialised:
 //
 //     C^T[n (TMEM lane), m (column)] = W^T[n][k] (A operand, TENSOR MEMORY) x op(A)^T[k][m] (B operand, shared memory)
 //
@@ -238,7 +75,7 @@ constexpr uint32_t T_WCOL = 256;                // W^T operand: TMEM columns [25
 // (N floats) per step, i.e. by compile-time immediates.  RS / AD / MZ say which operands exist (checked once, uniformly,
 // by the caller), so the loads of a batch are unconditional and issued back to back before the first use.
 template <int N, bool RS, bool AD, bool MZ, bool FULL>
-__device__ __forceinline__ void epi_rows(const Args& g, const uint32_t (&x)[32], size_t o0, float bias, int nrows) {
+__device__ __forceinline__ void epi_rows(const GemmArgs& g, const uint32_t (&x)[32], size_t o0, float bias, int nrows) {
   const float* rsp = g.resid + o0;
   const float* adp = g.add + o0;
   const float* mzp = g.mulz + o0;
@@ -265,13 +102,13 @@ __device__ __forceinline__ void epi_rows(const Args& g, const uint32_t (&x)[32],
   }
 }
 template <int N, bool RS, bool AD, bool MZ>
-__device__ __forceinline__ void epi_rows_any(const Args& g, const uint32_t (&x)[32], size_t o0, float bias, int nrows) {
+__device__ __forceinline__ void epi_rows_any(const GemmArgs& g, const uint32_t (&x)[32], size_t o0, float bias, int nrows) {
   if (nrows >= 32) epi_rows<N, RS, AD, MZ, true>(g, x, o0, bias, 32);
   else epi_rows<N, RS, AD, MZ, false>(g, x, o0, bias, nrows);
 }
 
 template <int K, int N>
-__global__ void __launch_bounds__(T_NT, 1) gemm_rows_tcT_kernel(const __grid_constant__ Args g) {
+__global__ void __launch_bounds__(T_NT, 1) gemm_rows_tcT_kernel(const __grid_constant__ GemmArgs g) {
   static_assert((K == 128 || K == 256) && (N == 128 || N == 256), "shapes");
   extern __shared__ __align__(1024) unsigned char smem[];
   __shared__ uint32_t tmem_slot;
@@ -462,30 +299,18 @@ __global__ void __launch_bounds__(T_NT, 1) gemm_rows_tcT_kernel(const __grid_con
 }
 
 template <int K, int N>
-cudaError_t launch(const Args& g, int num_sms, cudaStream_t st) {
+cudaError_t launch(const GemmArgs& g, int num_sms, cudaStream_t st) {
   const int ntiles = (g.M + 127) / 128;
   constexpr int NH = N / 128;
   int groups = num_sms / NH;
   if (groups > ntiles) groups = ntiles;
-  if (g.rowvec) {          // per-graph row vectors: only the staged kernel adds them
-    const size_t smem = (size_t)2 * 128 * K * sizeof(__nv_bfloat16) + (size_t)128 * STAGE_LD * sizeof(float);
-    auto kern = gemm_rows_tc_kernel<K, N>;
-    static bool configured = false;
-    if (!configured) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) return e;
-      configured = true;
-    }
-    kern<<<groups * NH, GEMM_NT, smem, st>>>(g);
-    return cudaGetLastError();
-  }
   const size_t smem = (size_t)T_NS * T_SLOT;
   auto kern = gemm_rows_tcT_kernel<K, N>;
-  static bool configuredT = false;
-  if (!configuredT) {
+  static bool configured = false;
+  if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    configuredT = true;
+    configured = true;
   }
   kern<<<groups * NH, T_NT, smem, st>>>(g);
   return cudaGetLastError();

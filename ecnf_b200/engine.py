@@ -199,7 +199,7 @@ class Engine:
         L.check(self.lib.ecnf_model_set_engine(self.handle, int(engine)), "ecnf_model_set_engine")
 
     def set_fm_chunk(self, graphs: int) -> None:
-        """Graphs per chunk of a training minibatch (gradients accumulate over the chunks); 0 = automatic."""
+        """Graphs per chunk of a training minibatch (gradients accumulate over the chunks); 0 = the whole minibatch."""
         L.check(self.lib.ecnf_model_set_fm_chunk(self.handle, int(graphs)), "ecnf_model_set_fm_chunk")
 
     @staticmethod

@@ -155,10 +155,9 @@ int ecnf_base_log_prob(const ecnf_model* m, const float* x, int64_t B, float* ou
  * out_loss: 1 float; out_grad: param_count floats in the parameter layout (sum over the B rows given,
  * already divided by `loss_denominator` = global_B * D so that shards add up under an all-reduce).         */
 int64_t ecnf_fm_workspace_bytes(const ecnf_model* m, int64_t B);
-/* A minibatch is processed in chunks of `graphs` graphs whose gradients accumulate (0 = automatic: the chunk's
- * [edge rows x mlp_units] fp32 activation matrices are sized to stay resident in the L2 between the kernel that writes
- * one and the kernel that reads it).  A per-handle attribute like the engine choice; changes the workspace size.  The
- * result is the same sum over rows in a different order (loss.py:25-31 is a mean over the batch).                  */
+/* A minibatch is processed in chunks of `graphs` graphs whose gradients accumulate (0, the default = the whole minibatch
+ * in one pass).  A per-handle attribute like the engine choice; changes the workspace size.  The result is the same sum
+ * over rows in a different order (loss.py:25-31 is a mean over the batch).                                           */
 int ecnf_model_set_fm_chunk(ecnf_model* m, int64_t graphs);
 int ecnf_fm_loss_grad(const ecnf_model* m, const float* x_data, const float* x0, const float* t,
                       const int32_t* feat, int64_t B, float loss_denominator, float* out_loss, float* out_grad,

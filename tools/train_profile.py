@@ -1,5 +1,5 @@
 """A few QM9-positional flow-matching steps (batch 512) for per-kernel timing under ncu (GPU box).
-Usage: python tools/train_profile.py [graphs per chunk, 0 = automatic]"""
+Usage: python tools/train_profile.py [graphs per chunk, 0 = the whole minibatch]"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import argparse
