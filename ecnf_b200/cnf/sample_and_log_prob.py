@@ -11,6 +11,12 @@ Differences, all documented in DESIGN.md:
     cannot run (sample_and_log_prob.py:140);
   * diffrax raises when max_steps (4096) is reached; the kernel flags the trajectory in its stats row, and the wrappers
     raise EcnfError from that flag by default (`check_status=False` skips the device->host read on hot paths).
+
+`ts=` is diffeqsolve's `saveat=SaveAt(ts=ts)` (at most 1024 times in [0, 1], in the direction of integration): the
+functions then also return the path, `xs` [B, n_save, D] and, in the log-density modes, `delta_ts` [B, n_save], the
+divergence integral from the start time to each ts[k].  Along a sample path log q_t(x_t) = log p0(x0) - delta_ts; along
+the get_log_prob path from the data x (t = 1) towards t = 0, log q_t(x_t) = log_p - delta_ts.  Interior times come from the
+Dopri5 dense output; the step sequence, and so every other output, is the same as without `ts`.
 """
 from typing import Optional, Tuple
 
@@ -54,8 +60,8 @@ def _jax_base_and_eps(eng, key, B: int, want_eps: bool):
 
 def sample_cnf(cnf: FlowMatchingCNF, params, key, features=None, use_fixed_step_size: bool = False,
                rtol: float = 1e-5, atol: float = 1e-5, step_size: float = 0.05, *, n_samples: Optional[int] = None,
-               x0=None, global_offset: int = 0, return_stats: bool = False, check_status: bool = True):
-    """ecnf/cnf/sample_and_log_prob.py:11-38."""
+               x0=None, global_offset: int = 0, return_stats: bool = False, check_status: bool = True, ts=None):
+    """ecnf/cnf/sample_and_log_prob.py:11-38: returns x1, or (x1, xs) with `ts=`."""
     eng = cnf.engine
     if x0 is not None:
         x0 = torch.as_tensor(x0, dtype=torch.float32, device=eng.device)
@@ -70,19 +76,25 @@ def sample_cnf(cnf: FlowMatchingCNF, params, key, features=None, use_fixed_step_
         else:
             x0 = eng.base_sample(key, B, global_offset)
     ctrl = L.make_ctrl(use_fixed_step_size, rtol, atol, step_size)
-    x1, _, stats = eng.solve(params, L.MODE_SAMPLE, x0, features, ctrl)
+    res = eng.solve(params, L.MODE_SAMPLE, x0, features, ctrl, ts=ts)
+    x1, stats = res[0], res[2]
     if check_status:
         eng.check_status(stats, "sample_cnf")
-    out = x1[0] if single else x1
-    return (out, stats) if return_stats else out
+    if ts is None:
+        out = x1[0] if single else x1
+        return (out, stats) if return_stats else out
+    xs = res[3]
+    out = (x1[0], xs[0]) if single else (x1, xs)
+    return (*out, stats) if return_stats else out
 
 
 def get_log_prob(cnf: FlowMatchingCNF, params, x, key=None, features=None, approx: bool = False,
                  use_fixed_step_size: bool = False, rtol: float = 1e-5, atol: float = 1e-5, step_size: float = 0.05,
                  *, eps=None, global_offset: int = 0, return_stats: bool = False,
-                 check_status: bool = True) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """ecnf/cnf/sample_and_log_prob.py:41-94: returns (log_p, log_prob_base, delta).  approx=True = the Hutchinson
-    branch (:69-78): one probe eps ~ N(0, I) per trajectory, drawn once from `key` (:55) -- or injected with `eps=`."""
+                 check_status: bool = True, ts=None) -> Tuple[torch.Tensor, ...]:
+    """ecnf/cnf/sample_and_log_prob.py:41-94: returns (log_p, log_prob_base, delta), + (xs, delta_ts) with `ts=` (times
+    decreasing from 1 towards 0).  approx=True = the Hutchinson branch (:69-78): one probe eps ~ N(0, I) per trajectory,
+    drawn once from `key` (:55) -- or injected with `eps=`."""
     eng = cnf.engine
     x = torch.as_tensor(x, dtype=torch.float32, device=eng.device)
     single = x.dim() == 1
@@ -96,18 +108,21 @@ def get_log_prob(cnf: FlowMatchingCNF, params, x, key=None, features=None, appro
             eps = torch.from_numpy(jr.normal_per_key(_jax_keys(key, x.shape[0]), eng.cfg.D)).to(eng.device)
         else:
             eps = eng.normal_noise(key, x.shape[0], global_offset, substream=1)
-    _, logs, stats = eng.solve(params, L.MODE_LOGPROB, x, features, ctrl, eps=eps if approx else None)
+    res = eng.solve(params, L.MODE_LOGPROB, x, features, ctrl, eps=eps if approx else None, ts=ts)
+    logs, stats = res[1], res[2]
     if check_status:
         eng.check_status(stats, "get_log_prob")
     out = (logs[0, 0], logs[0, 1], logs[0, 2]) if single else (logs[:, 0], logs[:, 1], logs[:, 2])
+    if ts is not None:
+        out = (*out, res[3][0], res[4][0]) if single else (*out, res[3], res[4])
     return (*out, stats) if return_stats else out
 
 
 def sample_and_log_prob_cnf(cnf: FlowMatchingCNF, params, key, features=None, approx: bool = False,
                             use_fixed_step_size: bool = False, rtol: float = 1e-5, atol: float = 1e-5,
                             step_size: float = 0.05, *, n_samples: Optional[int] = None, x0=None, eps=None,
-                            global_offset: int = 0, return_stats: bool = False, check_status: bool = True):
-    """ecnf/cnf/sample_and_log_prob.py:97-149: returns (x1, log_q).  approx=True = the Hutchinson branch (:123-133); the
+                            global_offset: int = 0, return_stats: bool = False, check_status: bool = True, ts=None):
+    """ecnf/cnf/sample_and_log_prob.py:97-149: returns (x1, log_q), + (xs, delta_ts) with `ts=`.  approx=True = the Hutchinson branch (:123-133); the
     reference draws its probe from the SAME key as the base sample (:130,137; SURVEY C#6), which here means the raw noise
     underneath `sample_base(key)` (substream 0) -- or inject it with `eps=`."""
     eng = cnf.engine
@@ -133,8 +148,11 @@ def sample_and_log_prob_cnf(cnf: FlowMatchingCNF, params, key, features=None, ap
             eps = torch.from_numpy(jr.normal_per_key(_jax_keys(key, x0.shape[0]), eng.cfg.D)).to(eng.device)
         else:
             eps = eng.normal_noise(key, x0.shape[0], global_offset, substream=0)
-    x1, logs, stats = eng.solve(params, L.MODE_SAMPLE_LOGQ, x0, features, ctrl, eps=eps if approx else None)
+    res = eng.solve(params, L.MODE_SAMPLE_LOGQ, x0, features, ctrl, eps=eps if approx else None, ts=ts)
+    x1, logs, stats = res[:3]
     if check_status:
         eng.check_status(stats, "sample_and_log_prob_cnf")
     out = (x1[0], logs[0, 0]) if single else (x1, logs[:, 0])
+    if ts is not None:
+        out = (*out, res[3][0], res[4][0]) if single else (*out, res[3], res[4])
     return (*out, stats) if return_stats else out

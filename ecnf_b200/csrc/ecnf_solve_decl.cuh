@@ -53,12 +53,18 @@ struct KernelArgs {
   TcImages img;
   TcSmemLayout lay;
   TcTabs tabs;
+  // SaveAt(ts) (kernels instantiated with SAVE only)
+  const float* ts;        // [n_save] internal (direction-multiplied) save times, increasing, in the workspace
+  int n_save;
+  float* out_traj;        // [B, n_save, D]
+  float* out_traj_delta;  // [B, n_save] (log-density modes)
 };
+static_assert(sizeof(KernelArgs) <= 4096, "KernelArgs is a by-value kernel parameter (4 KB limit)");
 
 // fp32 SIMT engine: its shape limits (ECNF_OK, or ECNF_ERR_UNSUPPORTED with the reason set), launch
 template <int U, int H, bool DIV>
 int simt_check(const ecnf_model* mdl);
-template <int U, int H, bool DIV>
+template <int U, int H, bool DIV, bool SAVE = false>
 int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st);
 
 // tensor-core engine ((U, H) = (128, 64) and (64, 32)): eligibility, extra workspace, launch
@@ -66,6 +72,6 @@ bool tc_eligible(const ecnf_model* mdl, bool div);
 int64_t tc_image_bytes(const ecnf_model* mdl);
 int64_t tc_flops_per_eval(const ecnf_model* mdl);
 int tc_tile_table(const ecnf_model* mdl, int kind, uint32_t* out, int64_t cap_words);
-int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bool div, cudaStream_t st);
+int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bool div, bool save, cudaStream_t st);
 
 }  // namespace ecnf_solve_detail

@@ -49,6 +49,15 @@ static __constant__ float c_BERR[7] = {(float)(35.0 / 384 - 1951.0 / 21600),
                                 (float)(-2187.0 / 6784 + 12231.0 / 42400),
                                 (float)(11.0 / 84 - 649.0 / 6300),
                                 (float)(-1.0 / 60)};
+// Dense output: y(t_mid) - y0 = sum_i c_MID[i] k_i, the midpoint weights of the Dopri5 4th-order interpolant as torchdiffeq and
+// diffrax carry them.  Recalled, like the b_hat above, not read from diffrax (DESIGN.md 3.1d).
+static __constant__ float c_MID[7] = {(float)(6025192743.0 / 30085553152.0 / 2),
+                               0.f,
+                               (float)(51252292925.0 / 65400821598.0 / 2),
+                               (float)(-2691868925.0 / 45128329728.0 / 2),
+                               (float)(187940372067.0 / 1594534317056.0 / 2),
+                               (float)(-1776094331.0 / 19743644256.0 / 2),
+                               (float)(11237099.0 / 235043384.0 / 2)};
 
 template <int U_, int H_>
 struct Geo {
@@ -615,7 +624,9 @@ __device__ __forceinline__ float clip_to_end(float tprev, float tnext, float T1,
 // The ODE driver (diffrax.diffeqsolve restated), generic over the engine that evaluates the vector field.
 // Written as a state machine around ONE call site of eng.eval so that the (large) evaluation code is inlined exactly
 // once and the engine's state stays in registers.
-template <class Eng, bool DIV>
+// SAVE: also write the path at the caller's times a.ts (diffrax SaveAt(ts)) from the Dopri5 dense output of each accepted
+// step.  A template parameter, so that the kernels without it keep their registers and spills.
+template <class Eng, bool DIV, bool SAVE>
 __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long long& s_traj, float* s_ctl) {
   const int tid = threadIdx.x;
   const int D = eng.D, S = DIV ? D + 1 : D;
@@ -676,6 +687,12 @@ __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long l
     const int32_t* feat = a.feat + b * eng.n;
     const float* xin = a.x_init + b * D;
     eng.set_eps(a.eps ? a.eps + b * D : nullptr);
+    // save row k, component i < S: positions to out_traj [B, n_save, D], the divergence integral to out_traj_delta [B, n_save]
+    auto put = [&](int k, int i, float v) {
+      if (i < D) a.out_traj[(b * a.n_save + k) * D + i] = v;
+      else a.out_traj_delta[b * a.n_save + k] = v;
+    };
+    int next_save = 0;   // first save time not yet written
 
     int phase, stage = 0, n_steps = 0, n_acc = 0, n_evals = 0, status = 0;
     float tprev = T0, tnext = T0, dt = 0.f, h0 = 0.f, d1 = 0.f, t_eval, lp0_start = 0.f;
@@ -693,6 +710,10 @@ __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long l
       ein = y;
     }
     __syncthreads();
+    if constexpr (SAVE) {   // a save time at the start time: the initial state, divergence integral 0
+      for (; next_save < a.n_save && a.ts[next_save] <= T0; ++next_save)
+        for (int i = tid; i < S; i += Eng::NT) put(next_save, i, y[i]);
+    }
     if (DIV && !vf_mode && !reverse) lp0_start = base_logp(y);   // log p0(x0), sample_and_log_prob.py:147
 
     bool running = true;
@@ -768,6 +789,33 @@ __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long l
           }
           new_prev = fminf(new_prev, T1);
           new_next = clip_to_end(new_prev, new_next, T1, keep);
+          if constexpr (SAVE) {
+            // every pending save time in (tprev, tnext] of this accepted step, from y0 = y, y1 = ys and k_0..k_6 (k_6 = dt F(tnext,
+            // y1), the FSAL stage): the Dopri5 4th-order interpolant (torchdiffeq _interp_fit), y1 itself at tnext.  Each thread
+            // reads the components of y it overwrites below, so no barrier is needed in between.
+            for (; keep && next_save < a.n_save && a.ts[next_save] <= tnext; ++next_save) {
+              const float tau_s = a.ts[next_save];
+              const bool at_end = !(tau_s < tnext);
+              const float sx = (tau_s - tprev) / dt;
+              for (int i = tid; i < S; i += Eng::NT) {
+                const float y0 = y[i], y1 = ys[i];
+                float v = y1;
+                if (!at_end) {
+                  const float k0 = kk[i], k6 = kk[6 * S + i];
+                  float ym = y0;
+                  for (int j = 0; j < 7; ++j) {
+                    const float cj = c_MID[j];
+                    if (cj != 0.f) ym = ym + cj * kk[j * S + i];
+                  }
+                  const float pa = 2.f * (k6 - k0) - 8.f * (y1 + y0) + 16.f * ym;
+                  const float pb = 5.f * k0 - 3.f * k6 + 18.f * y0 + 14.f * y1 - 32.f * ym;
+                  const float pc = k6 - 4.f * k0 - 11.f * y0 - 5.f * y1 + 16.f * ym;
+                  v = (((pa * sx + pb) * sx + pc) * sx + k0) * sx + y0;
+                }
+                put(next_save, i, v);
+              }
+            }
+          }
           if (keep) {
             for (int i = tid; i < S; i += Eng::NT) { y[i] = ys[i]; f0[i] = dir * fo[i]; }
             ++n_acc;
@@ -805,6 +853,10 @@ __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long l
       }
     }
     if (vf_mode) { __syncthreads(); continue; }
+    if constexpr (SAVE) {   // stopped on max_steps: NaN in the rows never reached
+      const int left = a.n_save - next_save;
+      for (int idx = tid; idx < left * S; idx += Eng::NT) put(next_save + idx / S, idx % S, __int_as_float(0x7fffffff));
+    }
 
     for (int i = tid; i < D; i += Eng::NT) a.out_x[b * D + i] = y[i];
     float lpb_end = 0.f;
@@ -831,13 +883,13 @@ __device__ __forceinline__ void solve_body(const KernelArgs& a, Eng& eng, long l
   }
 }
 
-template <int U, int H, bool DIV>
+template <int U, int H, bool DIV, bool SAVE>
 __global__ void __launch_bounds__(NTHREADS, 1) ecnf_solve_kernel(const __grid_constant__ KernelArgs a) {
   extern __shared__ __align__(16) float smem[];
   __shared__ long long s_traj;
   __shared__ float s_ctl[8];
   Engine<U, H, DIV> eng(a.m, smem, a.scratch + (size_t)blockIdx.x * a.scratch_stride, a.eps != nullptr);
-  solve_body<Engine<U, H, DIV>, DIV>(a, eng, s_traj, s_ctl);
+  solve_body<Engine<U, H, DIV>, DIV, SAVE>(a, eng, s_traj, s_ctl);
 }
 
 template <int U, int H, bool DIV>
@@ -857,12 +909,12 @@ int simt_check(const ecnf_model* mdl) {
   return ECNF_OK;
 }
 
-template <int U, int H, bool DIV>
+template <int U, int H, bool DIV, bool SAVE>
 int launch_t(const ecnf_model* mdl, KernelArgs& a, int grid, cudaStream_t st) {
   const int rc = simt_check<U, H, DIV>(mdl);
   if (rc != ECNF_OK) return rc;
   const size_t smem = (size_t)make_layout<U, H>(mdl->cfg.n_frames, mdl->cfg.dim, DIV).total_floats * sizeof(float);
-  auto kern = ecnf_solve_kernel<U, H, DIV>;
+  auto kern = ecnf_solve_kernel<U, H, DIV, SAVE>;
   ECNF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, NTHREADS, smem, st>>>(a);
   ECNF_CHECK_CUDA(cudaGetLastError());

@@ -1,0 +1,5 @@
+// Explicit instantiation of engine A for mlp_units=128, n_invariant_feat_hidden=64, exact divergence off, saving the path (SaveAt(ts)).
+#include "ecnf_solve_impl.cuh"
+namespace ecnf_solve_detail {
+template int launch_t<128, 64, false, true>(const ecnf_model*, KernelArgs&, int, cudaStream_t);
+}

@@ -64,9 +64,9 @@ TcTabs make_tabs(const ecnf_model* mdl, int MR, int ntan = 0) {   // ntan: 0 = n
 int64_t tables_bytes(const TcTabs& t) { return (int64_t)(t.off[TT_COUNT - 1] + t.cnt[TT_COUNT - 1]) * TC_TILE_WORDS * 4; }
 int64_t images_bytes(const ecnf_model* mdl) { return (walk_images(mdl, nullptr, nullptr) + 255) & ~255LL; }
 
-template <int U, int H, bool DIV>
+template <int U, int H, bool DIV, bool SAVE>
 int launch_one(const KernelArgs& a, int grid, size_t smem, cudaStream_t st) {
-  auto kern = ecnf_solve_tc_kernel<U, H, DIV>;
+  auto kern = ecnf_solve_tc_kernel<U, H, DIV, SAVE>;
   ECNF_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, TC_NT, smem, st>>>(a);
   ECNF_CHECK_CUDA(cudaGetLastError());
@@ -129,7 +129,7 @@ int tc_tile_table(const ecnf_model* mdl, int kind, uint32_t* out, int64_t cap_wo
   return cnt;
 }
 
-int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bool div, cudaStream_t st) {
+int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bool div, bool save, cudaStream_t st) {
   const ecnf_config& c = mdl->cfg;
   std::vector<TcPrepItem> items;
   a.img.base = reinterpret_cast<const unsigned char*>(image_ws);
@@ -153,9 +153,14 @@ int launch_tc(const ecnf_model* mdl, KernelArgs& a, int grid, void* image_ws, bo
   ECNF_CHECK_CUDA(cudaGetLastError());
   a.lay = layout_of(c, MR);
   const size_t smem = (size_t)a.lay.total_bytes;
+  if (save) {
+    if (c.mlp_units == 128)
+      return div ? launch_one<128, 64, true, true>(a, grid, smem, st) : launch_one<128, 64, false, true>(a, grid, smem, st);
+    return div ? launch_one<64, 32, true, true>(a, grid, smem, st) : launch_one<64, 32, false, true>(a, grid, smem, st);
+  }
   if (c.mlp_units == 128)
-    return div ? launch_one<128, 64, true>(a, grid, smem, st) : launch_one<128, 64, false>(a, grid, smem, st);
-  return div ? launch_one<64, 32, true>(a, grid, smem, st) : launch_one<64, 32, false>(a, grid, smem, st);
+    return div ? launch_one<128, 64, true, false>(a, grid, smem, st) : launch_one<128, 64, false, false>(a, grid, smem, st);
+  return div ? launch_one<64, 32, true, false>(a, grid, smem, st) : launch_one<64, 32, false, false>(a, grid, smem, st);
 }
 
 }  // namespace ecnf_solve_detail

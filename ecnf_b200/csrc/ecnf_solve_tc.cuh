@@ -1445,12 +1445,12 @@ struct EngineTC {
   }
 };
 
-template <int U, int H, bool DIV>
+template <int U, int H, bool DIV, bool SAVE>
 __global__ void __launch_bounds__(TC_NT, 1) ecnf_solve_tc_kernel(const __grid_constant__ KernelArgs a) {
   __shared__ long long s_traj;
   __shared__ float s_ctl[8];
   EngineTC<U, H, DIV> eng(a);
-  solve_body<EngineTC<U, H, DIV>, DIV>(a, eng, s_traj, s_ctl);
+  solve_body<EngineTC<U, H, DIV>, DIV, SAVE>(a, eng, s_traj, s_ctl);
   eng.finish(reinterpret_cast<long long*>(reinterpret_cast<char*>(a.counter) + 64));
 }
 

@@ -290,8 +290,12 @@ class Engine:
         return out
 
     # ---------------------------------------------------------------- ODE solves
-    def solve(self, params, mode: int, x_init, feat=None, ctrl: Optional[L.SolveCtrl] = None, eps=None):
-        """Returns (x_out [B, D], logs [B, 3] or None, stats int32 [B, 4]).  eps [B, D]: Hutchinson probes (approx=True)."""
+    def solve(self, params, mode: int, x_init, feat=None, ctrl: Optional[L.SolveCtrl] = None, eps=None, ts=None):
+        """Returns (x_out [B, D], logs [B, 3] or None, stats int32 [B, 4]).  eps [B, D]: Hutchinson probes (approx=True).
+
+        ts: save times (diffrax SaveAt(ts)), a 1-D sequence of floats in [0, 1], strictly increasing for the sample modes
+        and strictly decreasing for MODE_LOGPROB.  Then the result is (x_out, logs, stats, traj [B, n_save, D],
+        traj_delta [B, n_save] or None): the state and (log modes) the divergence integral at each time."""
         packed = self.pack(params)
         self._bind(packed)
         x_init, feat, B = self._prep(x_init, feat)
@@ -299,16 +303,29 @@ class Engine:
         out_x = torch.empty_like(x_init)
         logs = None if mode == L.MODE_SAMPLE else torch.empty(B, 3, dtype=torch.float32, device=self.device)
         stats = torch.empty(B, 4, dtype=torch.int32, device=self.device)
-        nb = int(self.lib.ecnf_solve_workspace_bytes(self.handle, mode, B))
-        ws = self._workspace("solve", nb)
         if eps is not None:
             eps = torch.as_tensor(eps, dtype=torch.float32, device=self.device).reshape(-1, self.cfg.D).contiguous()
             if eps.shape[0] != B or mode == L.MODE_SAMPLE:
                 raise L.EcnfError("Hutchinson probes need one row per trajectory and a log-density mode")
-        L.check(self.lib.ecnf_solve_hutchinson(self.handle, mode, _ptr(x_init), _ptr(feat), _ptr(eps), B, C.byref(ctrl),
-                                               _ptr(out_x), _ptr(logs), _ptr(stats), _ptr(ws), ws.numel(), _stream_ptr()),
-                "ecnf_solve_hutchinson")
-        return out_x, logs, stats
+        if ts is None:
+            nb = int(self.lib.ecnf_solve_workspace_bytes(self.handle, mode, B))
+            ws = self._workspace("solve", nb)
+            L.check(self.lib.ecnf_solve_hutchinson(self.handle, mode, _ptr(x_init), _ptr(feat), _ptr(eps), B,
+                                                   C.byref(ctrl), _ptr(out_x), _ptr(logs), _ptr(stats), _ptr(ws),
+                                                   ws.numel(), _stream_ptr()), "ecnf_solve_hutchinson")
+            return out_x, logs, stats
+        ts_host = np.ascontiguousarray(
+            (ts.detach().cpu().numpy() if isinstance(ts, torch.Tensor) else np.asarray(ts)).astype(np.float32).reshape(-1))
+        n_save = int(ts_host.size)
+        traj = torch.empty(B, n_save, self.cfg.D, dtype=torch.float32, device=self.device)
+        traj_delta = None if mode == L.MODE_SAMPLE else torch.empty(B, n_save, dtype=torch.float32, device=self.device)
+        nb = int(self.lib.ecnf_solve_saveat_workspace_bytes(self.handle, mode, B, n_save))
+        ws = self._workspace("solve", nb)
+        L.check(self.lib.ecnf_solve_saveat(self.handle, mode, _ptr(x_init), _ptr(feat), _ptr(eps), B, C.byref(ctrl),
+                                           n_save, ts_host.ctypes.data_as(C.POINTER(C.c_float)), _ptr(out_x), _ptr(logs),
+                                           _ptr(stats), _ptr(traj), _ptr(traj_delta), _ptr(ws), ws.numel(),
+                                           _stream_ptr()), "ecnf_solve_saveat")
+        return out_x, logs, stats, traj, traj_delta
 
     # ---------------------------------------------------------------- base distribution
     def base_sample(self, key, n: int, global_offset: int = 0) -> torch.Tensor:

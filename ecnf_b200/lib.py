@@ -15,6 +15,7 @@ PKG = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ["ECNF_B200_LIB"]) if os.environ.get("ECNF_B200_LIB") else PKG / "libecnf_b200.so"
 
 MODE_VF, MODE_VF_DIV, MODE_SAMPLE, MODE_SAMPLE_LOGQ, MODE_LOGPROB = range(5)
+MAX_SAVE_TIMES = 1024   # ECNF_MAX_SAVE_TIMES
 TARGET_LJ, TARGET_DW = 0, 1
 
 
@@ -70,6 +71,9 @@ SIGNATURES = {
     "ecnf_vf_forward_div": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I64, _P]),
     "ecnf_solve": (C.c_int, [_P, C.c_int, _P, _P, _I64, C.POINTER(SolveCtrl), _P, _P, _P, _P, _I64, _P]),
     "ecnf_solve_hutchinson": (C.c_int, [_P, C.c_int, _P, _P, _P, _I64, C.POINTER(SolveCtrl), _P, _P, _P, _P, _I64, _P]),
+    "ecnf_solve_saveat_workspace_bytes": (_I64, [_P, C.c_int, _I64, C.c_int]),
+    "ecnf_solve_saveat": (C.c_int, [_P, C.c_int, _P, _P, _P, _I64, C.POINTER(SolveCtrl), C.c_int, C.POINTER(_F), _P, _P, _P,
+                                    _P, _P, _P, _I64, _P]),
     "ecnf_vf_forward_hutchinson": (C.c_int, [_P, _P, _P, _P, _P, _I64, _P, _P, _P, _I64, _P]),
     "ecnf_normal_noise": (C.c_int, [_P, _U64, _I64, _I64, C.c_uint32, _P, _P]),
     "ecnf_base_sample": (C.c_int, [_P, _U64, _I64, _I64, _P, _P]),

@@ -137,6 +137,27 @@ int ecnf_solve_hutchinson(const ecnf_model* m, int mode, const float* x_init, co
                           int64_t B, const ecnf_solve_ctrl* ctrl, float* out_x, float* out_logs, int32_t* out_stats,
                           void* ws, int64_t ws_bytes, void* stream);
 
+/* ---- ODE solve that also reports the path: diffeqsolve(..., saveat=SaveAt(ts=ts)) at the same call sites
+ * (sample_and_log_prob.py:33-37,85-89,140-144).  ts_host is a HOST array of n_save (<= ECNF_MAX_SAVE_TIMES) fp32 times in
+ * [0, 1], strictly increasing for SAMPLE / SAMPLE_LOGQ and strictly decreasing for LOGPROB (the direction of integration);
+ * it is copied before the call returns.  Row k of the path is the joint state at ts[k]:
+ *   out_traj[b, k, :]    = x(ts[k])                                            [B, n_save, D] (vmap of a per-trajectory solve)
+ *   out_traj_delta[b, k] = the divergence integral accumulated from the start time to ts[k]   [B, n_save], log modes only
+ * so along a sample path log q_t(x_t) = log p0(x0) - out_traj_delta[b, k].  A time equal to the start time gives x_init and
+ * 0; a time equal to the end time gives out_x and out_logs[b, 2] bit for bit; an interior time comes from the Dopri5
+ * 4th-order dense output of the accepted step that contains it.  Saving does not change the step sequence: out_x,
+ * out_logs and out_stats are those of ecnf_solve_hutchinson.  A trajectory stopped on max_steps (status 1) has NaN in the
+ * rows it never reached.  n_save = 0: exactly ecnf_solve_hutchinson (ts_host / out_traj* unused).
+ * The workspace is ecnf_solve_saveat_workspace_bytes: ecnf_solve_workspace_bytes + the save-time table, rounded up to
+ * 256 B (the same value when n_save = 0).                                                                        */
+#define ECNF_MAX_SAVE_TIMES 1024
+int64_t ecnf_solve_saveat_workspace_bytes(const ecnf_model* m, int mode, int64_t B, int n_save);
+int ecnf_solve_saveat(const ecnf_model* m, int mode, const float* x_init, const int32_t* feat, const float* eps,
+                      int64_t B, const ecnf_solve_ctrl* ctrl, int n_save, const float* ts_host,
+                      float* out_x, float* out_logs, int32_t* out_stats,
+                      float* out_traj, float* out_traj_delta,
+                      void* ws, int64_t ws_bytes, void* stream);
+
 /* ---- base distribution (build_cnf.py:46-61, zero_com_base.py:44-47,64-93)                                */
 /* x0 = base_scale * remove_mean(eps); eps from a counter-based Philox4x32-10 stream keyed by
  * (seed, global sample index) so a sharded run reproduces the single-GPU draw.                             */

@@ -16,6 +16,7 @@
 //   * the workspace is an operand sized by the Python side with ecnf_*_workspace_bytes (the library never allocates);
 //   * a non-zero return code becomes ffi::Error::Internal(ecnf_last_error()).
 #include <cstdint>
+#include <vector>
 
 #include <cuda_runtime_api.h>
 
@@ -100,6 +101,34 @@ ffi::Error SolveHutchinsonImpl(cudaStream_t stream, int64_t model, int32_t mode,
                                       ws.untyped_data(), (int64_t)ws.size_bytes(), stream));
 }
 
+// jaxlib decodes an array attribute into a host ffi::Span<const T>.  The minimal header stand-in the syntax test compiles
+// against (tests/mock_xla) has no Span; there a vector, which has the same begin() / end(), takes its place.
+#ifdef XLA_FFI_API_FFI_H_
+using F32Array = ffi::Span<const float>;
+#else
+using F32Array = std::vector<float>;
+#endif
+
+// diffeqsolve(..., saveat=SaveAt(ts=ts)): the solve + the path at the times of the array attribute `ts`, which the library
+// copies into the workspace before returning (eps: the Hutchinson probes, or a zero-size operand for the exact trace;
+// out_traj_delta: a zero-size result in SAMPLE mode)
+ffi::Error SolveSaveatImpl(cudaStream_t stream, int64_t model, int32_t mode, int32_t fixed, float step_size, float rtol,
+                           float atol, float dtmin, int32_t max_steps, float err_scale, F32Array ts,
+                           ffi::Buffer<ffi::F32> params, ffi::Buffer<ffi::F32> x_init, ffi::Buffer<ffi::S32> feat,
+                           ffi::Buffer<ffi::F32> eps, ffi::Buffer<ffi::U8> ws, ffi::ResultBuffer<ffi::F32> out_x,
+                           ffi::ResultBuffer<ffi::F32> out_logs, ffi::ResultBuffer<ffi::S32> out_stats,
+                           ffi::ResultBuffer<ffi::F32> out_traj, ffi::ResultBuffer<ffi::F32> out_traj_delta) {
+  Bound b(model, params.typed_data());
+  const int64_t B = x_init.dimensions()[0];
+  const ecnf_solve_ctrl ctrl = Ctrl(fixed, step_size, rtol, atol, dtmin, max_steps, err_scale);
+  const std::vector<float> t(ts.begin(), ts.end());
+  return Status(ecnf_solve_saveat(b.m, mode, x_init.typed_data(), feat.typed_data(),
+                                  eps.element_count() ? eps.typed_data() : nullptr, B, &ctrl, (int)t.size(), t.data(),
+                                  out_x->typed_data(), out_logs->typed_data(), out_stats->typed_data(),
+                                  out_traj->typed_data(), out_traj_delta->typed_data(), ws.untyped_data(),
+                                  (int64_t)ws.size_bytes(), stream));
+}
+
 // x0 = base_scale * remove_mean(eps) with eps = jax.random.normal(key, ...) drawn on the JAX side  (zero_com_base.py:44-47)
 ffi::Error BaseSampleFromNoiseImpl(cudaStream_t stream, int64_t model, ffi::Buffer<ffi::F32> eps,
                                    ffi::ResultBuffer<ffi::F32> out_x0) {
@@ -177,6 +206,12 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(EcnfSolveHutchinson, SolveHutchinsonImpl,
                                   .Attr<float>("step_size").Attr<float>("rtol").Attr<float>("atol").Attr<float>("dtmin")
                                   .Attr<int32_t>("max_steps").Attr<float>("err_scale").Arg<F32>().Arg<F32>().Arg<S32>().Arg<F32>()
                                   .Arg<U8>().Ret<F32>().Ret<F32>().Ret<S32>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EcnfSolveSaveat, SolveSaveatImpl,
+                              ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("model").Attr<int32_t>("mode").Attr<int32_t>("fixed")
+                                  .Attr<float>("step_size").Attr<float>("rtol").Attr<float>("atol").Attr<float>("dtmin")
+                                  .Attr<int32_t>("max_steps").Attr<float>("err_scale").Attr<F32Array>("ts").Arg<F32>()
+                                  .Arg<F32>().Arg<S32>().Arg<F32>().Arg<U8>().Ret<F32>().Ret<F32>().Ret<S32>().Ret<F32>()
+                                  .Ret<F32>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(EcnfBaseSampleFromNoise, BaseSampleFromNoiseImpl,
                               ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("model").Arg<F32>().Ret<F32>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(EcnfBaseLogProb, BaseLogProbImpl,
