@@ -27,7 +27,8 @@ struct TcSmemLayout {
 };
 
 // tile tables of the tensor-core engine: which (group, slot) rows sit in which 8-column chunk (ecnf_solve_tc.cuh)
-enum { TT_NODE1 = 0, TT_NODE, TT_FIRST, TT_MID, TT_LAST, TT_EDGE1, TT_COUNT };   // *1: primal rows only (no divergence)
+// *1: primal rows only (no divergence); *_S: TT_NODE / TT_MID with the s shape-space tangents of the middle blocks
+enum { TT_NODE1 = 0, TT_NODE, TT_FIRST, TT_MID, TT_LAST, TT_EDGE1, TT_NODE_S, TT_MID_S, TT_COUNT };
 constexpr int TC_TILE_WORDS = 48;    // 32 chunk words (2 sub-tiles x 16 chunks) + 16 header words
 struct TcTabs {
   const uint32_t* base;

@@ -232,6 +232,26 @@ __host__ __device__ inline int tc_pack(int kind, int n, int dim, int SUB, int MR
   return tile;
 }
 
+// Tangent directions of the middle blocks on the shape-space path (DESIGN 3.1): s = D - dim - dim (dim - 1) / 2, the
+// centred directions orthogonal to the infinitesimal rotations of the evaluation's input.
+__host__ __device__ inline int tc_shape_tangents(int n, int dim) { return n * dim - dim - dim * (dim - 1) / 2; }
+// generator j of the rotations: the plane (p, q), p < q, in the order (0, 1), (0, 2), (1, 2); (A_j x)_p = x_q, (A_j x)_q = -x_p
+__host__ __device__ inline void tc_gen_pair(int j, int dim, int& p, int& q) {
+  p = 0;
+  while (j >= dim - 1 - p) { j -= dim - 1 - p; ++p; }
+  q = p + 1 + j;
+}
+// tc_pack for any table kind: the shape-space kinds TT_NODE_S / TT_MID_S are TT_NODE / TT_MID with ntan_s tangent rows
+// (no tiles when ntan_s < 1: the launch has no shape-space path)
+__host__ __device__ inline int tc_pack_kind(int kind, int n, int dim, int SUB, int MR, uint32_t* out, int ntan, int ntan_s,
+                                            uint32_t* stage = nullptr) {
+  if (kind == TT_NODE_S || kind == TT_MID_S) {
+    if (ntan_s < 1) return 0;
+    return tc_pack(kind == TT_NODE_S ? TT_NODE : TT_MID, n, dim, SUB, MR, out, ntan_s, stage);
+  }
+  return tc_pack(kind, n, dim, SUB, MR, out, ntan, stage);
+}
+
 // shared-memory carve-up; MR (rows of the message accumulator) is the largest 1 + 7k (<= ND) that fits in 227 KB
 template <int U, int H>
 __host__ __device__ inline TcSmemLayout make_tc_layout(int n, int dim, int MR) {
@@ -249,7 +269,7 @@ __host__ __device__ inline TcSmemLayout make_tc_layout(int n, int dim, int MR) {
   L.xs = take(D * 4);
   L.xs0 = take(D * 4);
   L.xacc = take(D * 4);
-  L.mu = take(16);
+  L.mu = take(32);     // the centroid (dim floats), then at word 4 the evaluation's tangent layout (EngineTC::tstate)
   L.tau = take(ECNF_MAX_T * 4);
   L.cvec = take(64 * 4);
   L.ode = take(11 * S * 4);
@@ -285,6 +305,243 @@ __host__ inline int tc_pick_mrows(int n, int dim, bool div) {
 
 extern __shared__ __align__(1024) unsigned char smem_tc[];
 
+// =====================================================================================================================
+// Shape-space tangents of the middle blocks (exact trace, DESIGN 3.1).  Every MLP input is E(n)-invariant and the
+// coordinate stream is equivariant, so along an infinitesimal rotation A_j x0 of the centred input the invariants have
+// zero tangent and the positions x^b have the tangent A_j x^b.  The middle blocks therefore carry only the s directions
+// q_k (columns of Q_S) orthogonal to translations and rotations; the canonical tangents P e_d are rebuilt before the
+// last block:  h-dot[P e_d] = sum_k Q_S[d,k] h-dot[q_k],   x-dot[P e_d] = sum_k Q_S[d,k] x-dot[q_k] + sum_j W[d,j] A_j x^b
+// with [A_j x0] = Q_R R_r (Householder QR of [translations | A_j x0]) and W = Q_R R_r^-T.
+// =====================================================================================================================
+// Free functions of plain arguments, called out of line (a member function would force the large inlined engine object
+// into local memory).  Callers: the 256 epilogue threads (named barrier 1).
+
+constexpr float TC_SHAPE_MIN_SIGMA = 0.05f;   // smallest singular value of [A_j x0] / |x0| of the shape-space path
+// the maps and the basis work in the two B-operand buffers (idle between the phases): floats available
+constexpr int TC_SHAPE_STAGE = 2 * TC_BOP / 4;
+// the shape-space path needs a map matrix (<= D x DP) and the tangent rows of one node (<= D x H) staged at once
+__host__ __device__ inline bool tc_shape_fits(int n, int dim, int H) {
+  const int D = n * dim, DP = (D + 7) & ~7;
+  return D * DP + D * H <= TC_SHAPE_STAGE;
+}
+
+// The basis of an evaluation's centred input xs; tstate[1] = s, or ntan (canonical path) when the rotations of xs are
+// (nearly) degenerate -- collinear or coincident particles.  V: fp64 shared-memory workspace (reflectors V [c][DP], the
+// reduced columns M [c][DP], Q_R [r][DP]); results QS = Q_S [D][SP] and QB = [Q_S^T ; W^T] [s + r][DP] (fp32, zero padded,
+// in the CTA's scratch).  fallbacks: profile counter or null.
+__device__ __noinline__ void tc_shape_basis(const float* xs, int n, int dim, int ntan, double* V, float* QS, float* QB,
+                                            int* tstate, long long* fallbacks) {
+  const int D = n * dim, r = dim * (dim - 1) / 2, c = dim + r, s = D - c, DP = (D + 7) & ~7, SP = (s + 7) & ~7;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  double* M = V + (size_t)c * DP;
+  double* QRd = M + (size_t)c * DP;
+  auto wsum = [](double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+  };
+  if (warp == 0) {
+    // M = [translations (unit, per coordinate) | A_j xs], column-major; Householder QR in place, reflectors
+    // v_j (|v_j|^2 = 2 or 0) to V
+    double xn2 = 0.0;
+    for (int row = lane; row < D; row += 32) {
+      const int i = row / dim, cc = row - i * dim;
+      xn2 += (double)xs[row] * (double)xs[row];
+      for (int j = 0; j < c; ++j) {
+        double v = 0.0;
+        if (j < dim) {
+          v = (cc == j) ? rsqrt((double)n) : 0.0;
+        } else {
+          int p, q;
+          tc_gen_pair(j - dim, dim, p, q);
+          v = cc == p ? (double)xs[i * dim + q] : cc == q ? -(double)xs[i * dim + p] : 0.0;
+        }
+        M[(size_t)j * DP + row] = v;
+      }
+    }
+    xn2 = wsum(xn2);
+    __syncwarp();
+    for (int j = 0; j < c; ++j) {
+      double nx = 0.0;
+      for (int row = j + lane; row < D; row += 32) nx += M[(size_t)j * DP + row] * M[(size_t)j * DP + row];
+      nx = wsum(nx);
+      const double xj = M[(size_t)j * DP + j];
+      const double alpha = xj > 0.0 ? -sqrt(nx) : sqrt(nx);
+      const double vv = nx - xj * xj + (xj - alpha) * (xj - alpha);
+      const double sc = vv > 0.0 ? sqrt(2.0 / vv) : 0.0;
+      for (int row = lane; row < D; row += 32)
+        V[(size_t)j * DP + row] = row < j ? 0.0 : sc * (row == j ? xj - alpha : M[(size_t)j * DP + row]);
+      __syncwarp();
+      for (int l = j; l < c; ++l) {
+        double d = 0.0;
+        for (int row = j + lane; row < D; row += 32) d += V[(size_t)j * DP + row] * M[(size_t)l * DP + row];
+        d = wsum(d);
+        for (int row = j + lane; row < D; row += 32) M[(size_t)l * DP + row] -= d * V[(size_t)j * DP + row];
+        __syncwarp();
+      }
+    }
+    if (lane == 0) {
+      // smallest eigenvalue of the Gram matrix R_r^T R_r of the rotation columns (R_r = M[dim + b][dim + a], a <= b)
+      auto R = [&](int a2, int b2) { return a2 <= b2 ? M[(size_t)(dim + b2) * DP + dim + a2] : 0.0; };
+      double lmin = 0.0;
+      if (r == 1) {
+        lmin = R(0, 0) * R(0, 0);
+      } else if (r == 3) {
+        double g[3][3];
+        for (int a2 = 0; a2 < 3; ++a2)
+          for (int b2 = 0; b2 < 3; ++b2) {
+            double v = 0.0;
+            for (int k = 0; k < 3; ++k) v += R(k, a2) * R(k, b2);
+            g[a2][b2] = v;
+          }
+        const double p1 = g[0][1] * g[0][1] + g[0][2] * g[0][2] + g[1][2] * g[1][2];
+        const double qm = (g[0][0] + g[1][1] + g[2][2]) / 3.0;
+        const double b0 = g[0][0] - qm, b1 = g[1][1] - qm, b2 = g[2][2] - qm;
+        const double p2 = b0 * b0 + b1 * b1 + b2 * b2 + 2.0 * p1;
+        if (p2 <= 0.0) {
+          lmin = qm;
+        } else {
+          const double pp = sqrt(p2 / 6.0);
+          const double det = b0 * (b1 * b2 - g[1][2] * g[1][2]) - g[0][1] * (g[0][1] * b2 - g[1][2] * g[0][2]) +
+                             g[0][2] * (g[0][1] * g[1][2] - b1 * g[0][2]);
+          const double hr = fmin(1.0, fmax(-1.0, det / (2.0 * pp * pp * pp)));
+          lmin = qm + 2.0 * pp * cos(acos(hr) / 3.0 + 2.0943951023931957);
+        }
+      }
+      const double thr = (double)TC_SHAPE_MIN_SIGMA * TC_SHAPE_MIN_SIGMA * xn2;
+      const bool ok = s >= 1 && xn2 > 0.0 && (r == 0 || lmin > thr);
+      tstate[1] = ok ? s : ntan;
+      if (!ok && fallbacks) *fallbacks += 1;
+    }
+  }
+  named_bar_sync(1, TC_EPI);
+  if (tstate[1] == ntan) return;
+  // Q e_k = H_0 ... H_{c-1} e_k for k >= dim, a warp per column: Q_R (k < c) to QRd, Q_S (k >= c) to QS and QB
+  for (int k = dim + warp; k < D; k += TC_EPI / 32) {
+    double w[8];      // rows lane + 32 u (D <= 255)
+#pragma unroll
+    for (int u = 0; u < 8; ++u) w[u] = (lane + 32 * u == k) ? 1.0 : 0.0;
+    for (int j = c - 1; j >= 0; --j) {
+      double d = 0.0;
+#pragma unroll
+      for (int u = 0; u < 8; ++u)
+        if (lane + 32 * u < D) d += V[(size_t)j * DP + lane + 32 * u] * w[u];
+      d = wsum(d);
+#pragma unroll
+      for (int u = 0; u < 8; ++u)
+        if (lane + 32 * u < D) w[u] -= d * V[(size_t)j * DP + lane + 32 * u];
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int row = lane + 32 * u;
+      if (row >= D) continue;
+      if (k < c) {
+        QRd[(size_t)(k - dim) * DP + row] = w[u];
+      } else {
+        QS[(size_t)row * SP + (k - c)] = (float)w[u];
+        QB[(size_t)(k - c) * DP + row] = (float)w[u];
+      }
+    }
+  }
+  // zero padding of QS (columns [s, SP)) and of QB's rows (columns [D, DP))
+  for (int idx = tid; idx < D * (SP - s); idx += TC_EPI) QS[(size_t)(idx / (SP - s)) * SP + s + idx % (SP - s)] = 0.f;
+  for (int idx = tid; idx < (s + r) * (DP - D); idx += TC_EPI) QB[(size_t)(idx / (DP - D)) * DP + D + idx % (DP - D)] = 0.f;
+  named_bar_sync(1, TC_EPI);
+  // W = Q_R R_r^-T: per row d, R_r W[d]^T = Q_R[d]^T by back substitution -> the rows s .. s + r - 1 of QB
+  for (int d = tid; d < D; d += TC_EPI) {
+    double wv[3];
+    for (int mm = r - 1; mm >= 0; --mm) {
+      double v = QRd[(size_t)mm * DP + d];
+      for (int b2 = mm + 1; b2 < r; ++b2) v -= M[(size_t)(dim + b2) * DP + dim + mm] * wv[b2];
+      wv[mm] = v / M[(size_t)(dim + mm) * DP + dim + mm];
+      QB[(size_t)(s + mm) * DP + d] = (float)wv[mm];
+    }
+  }
+  named_bar_sync(1, TC_EPI);
+}
+
+// global -> shared, nfloats (a multiple of 4, both ends 16-byte aligned) by asynchronous 16-byte copies of the epilogue
+// threads: complete after cp_async_wait and a barrier
+__device__ __forceinline__ void tc_stage(float* dst, const float* src, int nfloats) {
+  for (int c = threadIdx.x; c < nfloats / 4; c += TC_EPI) cp_async16(dst + 4 * c, src + 4 * c);
+}
+
+// h[i][1 + o] = sum_k Mx[k][o] h[i][1 + k] (o < no, k < nk) for every node (h rows of H floats, slot stride ND; Mx
+// row-major [nk][MP], MP a multiple of 8, zero beyond no).  Mx and the tangent rows of as many nodes as fit are staged in
+// `stage` (shared memory, TC_SHAPE_STAGE floats), so h is rewritten in place.
+template <int H>
+__device__ __noinline__ void tc_map_h(float* h, float* stage, const float* Mx, int n, int ND, int nk, int no, int MP) {
+  constexpr int NG = TC_EPI / H;
+  const int tid = threadIdx.x, fh = tid % H, nob = (no + 7) >> 3, per = nk * H;
+  float* hs = stage + nk * MP;
+  const int nn = (TC_SHAPE_STAGE - nk * MP) / per;
+  tc_stage(stage, Mx, nk * MP);
+  for (int i0 = 0; i0 < n; i0 += nn) {
+    const int ni = min(nn, n - i0);
+    for (int il = 0; il < ni; ++il) tc_stage(hs + il * per, h + ((size_t)(i0 + il) * ND + 1) * H, per);
+    cp_async_commit();
+    cp_async_wait<0>();
+    named_bar_sync(1, TC_EPI);
+    for (int task = tid / H; task < ni * nob; task += NG) {
+      const int il = task / nob, o0 = 8 * (task - il * nob);
+      const float* sp = hs + il * per + fh;
+      float acc[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) acc[u] = 0.f;
+#pragma unroll 4
+      for (int k = 0; k < nk; ++k) {
+        const float x = sp[k * H];
+        const float4 m0 = *reinterpret_cast<const float4*>(stage + k * MP + o0);
+        const float4 m1 = *reinterpret_cast<const float4*>(stage + k * MP + o0 + 4);
+        acc[0] = fmaf(x, m0.x, acc[0]); acc[1] = fmaf(x, m0.y, acc[1]); acc[2] = fmaf(x, m0.z, acc[2]); acc[3] = fmaf(x, m0.w, acc[3]);
+        acc[4] = fmaf(x, m1.x, acc[4]); acc[5] = fmaf(x, m1.y, acc[5]); acc[6] = fmaf(x, m1.z, acc[6]); acc[7] = fmaf(x, m1.w, acc[7]);
+      }
+      float* dp = h + ((size_t)(i0 + il) * ND + 1 + o0) * H + fh;
+#pragma unroll
+      for (int u = 0; u < 8; ++u)
+        if (o0 + u < no) dp[(size_t)u * H] = acc[u];
+    }
+    named_bar_sync(1, TC_EPI);
+  }
+}
+// xt[row][o] (stride no) = sum_{k < nk} xt[row][k] Mx[k][o] (stride nk) + (rot) sum_j (A_j xs)[row] Mx[nk + j][o],
+// through xtacc
+__device__ __noinline__ void tc_map_xt(float* xt, float* xtacc, const float* xs, const float* Mx_g, float* stage, int D, int dim,
+                                       int nk, int no, int MP, bool rot) {
+  const int tid = threadIdx.x, nob = (no + 7) >> 3, r = rot ? dim * (dim - 1) / 2 : 0;
+  const float* Mx = stage;
+  tc_stage(stage, Mx_g, (nk + r) * MP);
+  cp_async_commit();
+  cp_async_wait<0>();
+  named_bar_sync(1, TC_EPI);
+  for (int task = tid; task < D * nob; task += TC_EPI) {
+    const int row = task / nob, o0 = 8 * (task - row * nob), i = row / dim, cc = row - i * dim;
+    float acc[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) acc[u] = 0.f;
+    for (int k = 0; k < nk + r; ++k) {
+      float x;
+      if (k < nk) {
+        x = xt[row * nk + k];
+      } else {
+        int p, q;
+        tc_gen_pair(k - nk, dim, p, q);
+        x = cc == p ? xs[i * dim + q] : cc == q ? -xs[i * dim + p] : 0.f;
+      }
+      const float4 m0 = *reinterpret_cast<const float4*>(Mx + (size_t)k * MP + o0);
+      const float4 m1 = *reinterpret_cast<const float4*>(Mx + (size_t)k * MP + o0 + 4);
+      acc[0] = fmaf(x, m0.x, acc[0]); acc[1] = fmaf(x, m0.y, acc[1]); acc[2] = fmaf(x, m0.z, acc[2]); acc[3] = fmaf(x, m0.w, acc[3]);
+      acc[4] = fmaf(x, m1.x, acc[4]); acc[5] = fmaf(x, m1.y, acc[5]); acc[6] = fmaf(x, m1.z, acc[6]); acc[7] = fmaf(x, m1.w, acc[7]);
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u)
+      if (o0 + u < no) xtacc[row * no + o0 + u] = acc[u];
+  }
+  named_bar_sync(1, TC_EPI);
+  for (int idx = tid; idx < D * no; idx += TC_EPI) xt[idx] = xtacc[idx];
+  named_bar_sync(1, TC_EPI);
+}
+
 // Every buffer is addressed as (shared-memory base + offset from the kernel parameters): the offsets are constant-bank
 // loads, so no pointer has to be kept alive in (or spilled from) registers across the very large inlined body.
 #define TCF(field) (reinterpret_cast<float*>(smem_tc + a.lay.field))
@@ -298,6 +555,9 @@ struct EngineTC {
   static constexpr int NT = TC_NT;
   static constexpr int KN = SUB * H;      // K of the node-level layers (h rows of both sub-tiles)
   static constexpr int ROWB = 4 * H;      // bytes of one pre-split h_in row: H bf16 hi | H bf16 lo
+  // the shape-space path of the middle blocks is compiled for the (128, 64) network only: the (64, 32) kernel is left as
+  // it was (with the path compiled in, it ran 7 % slower on the canonical tables it keeps, DESIGN 3.1)
+  static constexpr bool SHAPE = DIV && U_ == 128;
   const KernelArgs& a;     // the __grid_constant__ kernel parameter
   const EcnfModelDev& m;
   const TcImages& img;
@@ -312,7 +572,8 @@ struct EngineTC {
 
   enum { B_READY = 0, B_DONE = 1, B_BUILT = 2, B_HEADS = 3, B_BFREE = 4 };
   enum { P_NODE_PRE, P_EDGE, P_NODE_POST, P_WAIT, P_EPI, P_MSG, P_HEAD, P_WLOAD, P_SIDE_WAIT, P_SIDE_GATHER, P_SIDE_COORD,
-         P_SIDE_META, P_SIDE_CPWAIT, P_NBUILD, P_NCOUNT };
+         P_SIDE_META, P_SIDE_CPWAIT, P_NBUILD, P_SHAPE /* basis + the two maps */, P_FALLBACK /* evaluations, not cycles */,
+         P_NCOUNT };
 #ifdef ECNF_TC_PROFILE
   long long prof_t0, prof_t1;
   __device__ __forceinline__ long long* prof_s() const { return reinterpret_cast<long long*>(smem_tc + a.lay.prof); }
@@ -339,6 +600,17 @@ struct EngineTC {
   __device__ __forceinline__ float* Mg() const { return hB() + (size_t)n * ND * H; }
   __device__ __forceinline__ float* Ph() const { return Mg() + (size_t)n * ND * U; }
   __device__ __forceinline__ unsigned char* Himg() const { return reinterpret_cast<unsigned char*>(Ph() + (size_t)n * ND * U); }
+  // the evaluation's shape-space basis (exact trace), in the spare tail of the scratch behind the h_in image (the SIMT
+  // engine's P_s / P_r space; tc_eligible checks that it fits): QS = Q_S [D][SP] and QB = [Q_S^T ; W^T] [s + r][DP]
+  // (DP, SP: D, s rounded up to 8, zero padded)
+  __device__ __forceinline__ float* basisQS() const { return reinterpret_cast<float*>(Himg() + ((size_t)n * ND + 1) * ROWB); }
+  __device__ __forceinline__ float* basisQB() const {
+    const int s = tc_shape_tangents(n, dim), SP = (s + 7) & ~7;
+    return basisQS() + (size_t)D * SP;
+  }
+  // the tangent layout of the evaluation (shared memory, beside the centroid): [0] the directions the running block
+  // carries = the row stride of xt / xtacc, [1] the directions of the middle blocks (s on the shape-space path, else ntan)
+  __device__ __forceinline__ int* tstate() const { return reinterpret_cast<int*>(smem_tc + a.lay.mu) + 4; }
 
   __device__ __forceinline__ EngineTC(const KernelArgs& a_)
       : a(a_), m(a_.m), img(a_.img), hutch(DIV && a_.eps != nullptr), n(a_.m.n), dim(a_.m.dim), D(a_.m.n * a_.m.dim),
@@ -958,7 +1230,9 @@ struct EngineTC {
     static constexpr bool side_build = true;
     __device__ __forceinline__ uint32_t a_col(int q, int) const { return TC_WCOL + 128u * (q & 1); }
     __device__ __forceinline__ int K(int) const { return 128; }
-    __device__ __forceinline__ int ekind() const { return kind == TT_FIRST ? KIND_FIRST : kind == TT_MID ? KIND_MID : KIND_LAST; }   // TT_EDGE1 has no tangent columns: the value is never used
+    __device__ __forceinline__ int ekind() const {
+      return kind == TT_FIRST ? KIND_FIRST : (kind == TT_MID || kind == TT_MID_S) ? KIND_MID : KIND_LAST;
+    }   // TT_EDGE1 has no tangent columns: the value is never used
     __device__ __forceinline__ int wimg(int w) const {
       const TcImgBlock& ib = e.img.blk[b];
       const int L = e.m.L;
@@ -976,7 +1250,7 @@ struct EngineTC {
       }
       for (int i = e.tid; i < D; i += NTH) { TCF(xacc)[i] = 0.f; TCF(dacc)[i] = 0.f; }
       if (DIV && kind != TT_LAST)
-        for (int i = e.tid; i < D * e.ntan; i += NTH) TCF(xtacc)[i] = 0.f;
+        for (int i = e.tid; i < D * (SHAPE ? e.tstate()[0] : e.ntan); i += NTH) TCF(xtacc)[i] = 0.f;
       if (want_msg)
         for (int i = e.tid; i < 2 * SUB * (a.lay.mrows + 1) * U; i += NTH) TCF(macc)[i] = 0.f;
       // per-edge geometry (egnn.py:73)
@@ -1036,7 +1310,7 @@ struct EngineTC {
     // per-column tables of `tile` for the epilogue threads: |v|^2 (or its tangent), message-accumulator row
     __device__ __forceinline__ void side_meta(int tb, int tile) {
       const KernelArgs& a = e.a;
-      const int sc = e.tid - TC_EPI, n = e.n, dim = e.dim, D = e.D, ND = e.ND;
+      const int sc = e.tid - TC_EPI, n = e.n, dim = e.dim, D = e.D, ND = e.ND, xts = SHAPE ? e.tstate()[0] : e.ntan;
       const uint32_t* tp = e.tile_ptr(kind, tile);
       const int win_i = (int)__ldg(tp + 32 + TH_WIN_I), win_s = (int)__ldg(tp + 32 + TH_WIN_S), win_ns = (int)__ldg(tp + 32 + TH_WIN_NS);
       const int dump = a.lay.mrows * U;
@@ -1062,7 +1336,7 @@ struct EngineTC {
             float acc = 0.f;
 #pragma unroll
             for (int cc = 0; cc < 3; ++cc)
-              if (cc < dim) acc = fmaf(gv[cc], TCF(xt)[(i * dim + cc) * e.ntan + k] - TCF(xt)[(j * dim + cc) * e.ntan + k], acc);
+              if (cc < dim) acc = fmaf(gv[cc], TCF(xt)[(i * dim + cc) * xts + k] - TCF(xt)[(j * dim + cc) * xts + k], acc);
             sd = isz ? 0.f : 2.f * acc;
           }
           if (want_msg && !((c & 7) == 0 && DIV && !(cw & CH_OWNER))) {      // a repeated primal column contributes nothing
@@ -1090,7 +1364,7 @@ struct EngineTC {
     __device__ __forceinline__ void side_coords(int tb, int tile) {
       const KernelArgs& a = e.a;
       const EcnfBlockParams& bp = e.m.blk[b];
-      const int sc = e.tid - TC_EPI, n = e.n, dim = e.dim, D = e.D;
+      const int sc = e.tid - TC_EPI, n = e.n, dim = e.dim, D = e.D, xts = SHAPE ? e.tstate()[0] : e.ntan;
       const int ek = ekind();
       const float bpv = bp.bp[0];
       float* cd = TCF(cdbuf);
@@ -1122,7 +1396,7 @@ struct EngineTC {
             for (int cc = 0; cc < 3; ++cc) {
               if (cc < dim) {
                 const float vc = gv[cc];
-                const float vd = TCF(xt)[(i * dim + cc) * e.ntan + k] - TCF(xt)[(j * dim + cc) * e.ntan + k];
+                const float vd = TCF(xt)[(i * dim + cc) * xts + k] - TCF(xt)[(j * dim + cc) * xts + k];
                 val[cc] = (pdv * vc + pg * vd) * inv - pg * vc * ld * inv * inv;
               }
             }
@@ -1184,7 +1458,7 @@ struct EngineTC {
           } while (q >= 0 && !(TCW(chw)[tb * 32 + widx(q)] & CH_RUNEND));
           if (u == 0) TCF(xacc)[i * dim + cc] += acc;
           else if (ek == KIND_LAST) TCF(dacc)[i * dim + cc] += acc;
-          else TCF(xtacc)[(i * dim + cc) * e.ntan + (ek == KIND_MID ? ch_qb(cw) + u - 2 : i * dim + (u - 1))] += acc;
+          else TCF(xtacc)[(i * dim + cc) * xts + (ek == KIND_MID ? ch_qb(cw) + u - 2 : i * dim + (u - 1))] += acc;
         }
       }
       e.side_bar();      // cdbuf is rewritten by the next tile
@@ -1345,6 +1619,33 @@ struct EngineTC {
     }
   };
 
+  // ---- shape-space tangents of the middle blocks (exact trace; tc_shape_basis, tc_map_h, tc_map_xt) ----
+  // epilogue threads: the basis of this evaluation's centred input xs; tstate()[1] = s, or ntan (canonical path)
+  __device__ __forceinline__ void shape_basis() {
+#ifdef ECNF_TC_PROFILE
+    long long* fb = prof_s() + P_FALLBACK;
+#else
+    long long* fb = nullptr;
+#endif
+    tc_shape_basis(TCF(xs), n, dim, ntan, reinterpret_cast<double*>(smem_tc + a.lay.bop), basisQS(), basisQB(), tstate(), fb);
+  }
+  // after block 0: h and xt from the canonical directions P e_d to the shape directions q_k
+  __device__ __forceinline__ void to_shape(int s) {
+    const int SP = (s + 7) & ~7;
+    tc_map_h<H>(hA(), TCF(bop), basisQS(), n, ND, D, s, SP);
+    tc_map_xt(TCF(xt), TCF(xtacc), TCF(xs), basisQS(), TCF(bop), D, dim, D, s, SP, false);
+    if (tid == 0) tstate()[0] = s;
+    epi_bar();
+  }
+  // before the last block: back to the canonical directions (the rotation part of xt from the positions xs = x^b)
+  __device__ __forceinline__ void to_canonical(int s) {
+    const int DP = (D + 7) & ~7;
+    tc_map_h<H>(hA(), TCF(bop), basisQB(), n, ND, s, D, DP);
+    tc_map_xt(TCF(xt), TCF(xtacc), TCF(xs), basisQB(), TCF(bop), D, dim, s, D, DP, true);
+    if (tid == 0) tstate()[0] = D;
+    epi_bar();
+  }
+
   // ---- one evaluation of (f, div f) at time t for the positions in xin (shared memory, D floats) ----
   __device__ __forceinline__ void eval(float t, const float* xin, const int32_t* feat, float* fout) {
     if (is_epi) {
@@ -1389,17 +1690,27 @@ struct EngineTC {
         ft = max(0, min(m.nfeat - 1, ft));
         h0[(size_t)node * ND * H + col] = m.embed[ft * H + col];
       }
+      if constexpr (SHAPE)
+        if (tid == 0) { tstate()[0] = ntan; tstate()[1] = ntan; }
       epi_bar();
+      if constexpr (SHAPE) {
+        // the shape-space tables exist only for the exact trace with middle blocks (launch_tc)
+        if (a.tabs.cnt[TT_MID_S] > 0 && m.nblocks >= 3) { qbeg(); shape_basis(); qend(P_SHAPE); }
+      }
     }
 #pragma unroll 1
     for (int b = 0; b < m.nblocks; ++b) {
       const bool last = (b == m.nblocks - 1);
       const bool htan = DIV && b > 0;
-      const int ekind = !DIV ? TT_EDGE1 : hutch ? TT_MID : last ? TT_LAST : (b == 0 ? TT_FIRST : TT_MID);
-      const int nkind = DIV ? TT_NODE : TT_NODE1;
+      // a middle block of the exact trace on the shape-space path (tstate: the layout chosen by shape_basis, whose
+      // epilogue barrier precedes every barrier arrival this thread has waited on since)
+      bool shape = false;
+      if constexpr (SHAPE) shape = b > 0 && !last && tstate()[1] < ntan;
+      const int ekind = !DIV ? TT_EDGE1 : hutch ? TT_MID : last ? TT_LAST : b == 0 ? TT_FIRST : shape ? TT_MID_S : TT_MID;
+      const int nkind = !DIV ? TT_NODE1 : shape ? TT_NODE_S : TT_NODE;
       pbeg();
       if (!is_side) {
-        const int kind = htan ? TT_NODE : TT_NODE1;
+        const int kind = !htan ? TT_NODE1 : shape ? TT_NODE_S : TT_NODE;
         NodePre p{*this, b, a.tabs.cnt[kind], last ? 1 : 2, kind};
         run_phase(p);
       }
@@ -1419,8 +1730,21 @@ struct EngineTC {
         epi_bar();
         const float invnb = 1.f / (float)(n - 1);
         for (int i = tid; i < D; i += TC_EPI) TCF(xs)[i] += TCF(xacc)[i] * invnb;
-        if (DIV && (!last || hutch))
-          for (int i = tid; i < D * ntan; i += TC_EPI) TCF(xt)[i] += TCF(xtacc)[i] * invnb;
+        if constexpr (DIV) {
+          const int xts = SHAPE ? tstate()[0] : ntan;
+          if (!last || hutch)
+            for (int i = tid; i < D * xts; i += TC_EPI) TCF(xt)[i] += TCF(xtacc)[i] * invnb;
+        }
+        if constexpr (SHAPE) {
+          const int ns = tstate()[1];
+          if (ns < ntan && (b == 0 || b == m.nblocks - 2)) {
+            epi_bar();
+            qbeg();
+            if (b == 0) to_shape(ns);
+            else to_canonical(ns);
+            qend(P_SHAPE);
+          }
+        }
       }
       if (is_epi || is_side) phase_bar();
       pend(P_NODE_POST);
@@ -1492,10 +1816,12 @@ __global__ void tc_prep_kernel(const float* __restrict__ params, unsigned char* 
 }
 
 // one CTA per table kind (a single thread packs: the work is sequential), the current tile staged in shared memory
-__global__ void tc_tables_kernel(uint32_t* __restrict__ out, int n, int dim, int SUB, int MR, int ntan, TcTabs tabs) {
+// ntan_s: tangent rows of the shape-space kinds (0: none)
+__global__ void tc_tables_kernel(uint32_t* __restrict__ out, int n, int dim, int SUB, int MR, int ntan, int ntan_s, TcTabs tabs) {
   __shared__ uint32_t stage[TC_TILE_WORDS];
   const int k = blockIdx.x;
-  if (threadIdx.x == 0 && k < TT_COUNT) tc_pack(k, n, dim, SUB, MR, out + (size_t)tabs.off[k] * TC_TILE_WORDS, ntan, stage);
+  if (threadIdx.x == 0 && k < TT_COUNT)
+    tc_pack_kind(k, n, dim, SUB, MR, out + (size_t)tabs.off[k] * TC_TILE_WORDS, ntan, ntan_s, stage);
 }
 
 #undef TCF

@@ -13,7 +13,9 @@ from ecnf_b200.nets.egnn import init_flat_params
 
 # epilogue thread 0: phases + its own time inside the edge phase; side thread 0: its own loop
 NAMES = ["node_pre", "edge", "node_post", "  epi: wait_mma", "  epi: chain (ld+act+split+st)", "  epi: messages", "  epi: head dot", "  epi: weight_load",
-         "  side: wait_heads", "  side: gather issue", "  side: coords", "  side: meta", "  side: copy wait + arrive", "  epi: node build"]
+         "  side: wait_heads", "  side: gather issue", "  side: coords", "  side: meta", "  side: copy wait + arrive", "  epi: node build",
+         "  epi: shape basis + maps"]
+NFALLBACK = len(NAMES)    # the next counter: evaluations of CTA 0 on the canonical path (degenerate rotations), not cycles
 NTOP = 3
 name = sys.argv[1] if len(sys.argv) > 1 else "lj13"
 B = int(sys.argv[2]) if len(sys.argv) > 2 else 148
@@ -33,9 +35,10 @@ for it in range(2):
     torch.cuda.synchronize()
     ms = a.elapsed_time(b)
 ws = next(v for k, v in eng._ws.items() if k[0] == "solve")
-prof = ws[64:64 + 8 * len(NAMES)].view(torch.int64).cpu().numpy()
+prof = ws[64:64 + 8 * (len(NAMES) + 1)].view(torch.int64).cpu().numpy()
 evals = int(stats[:, 2].sum()) / min(B, 148)
 tot = prof[:NTOP].sum()
 print(f"{name} B={B} kernel {ms:.1f} ms ({B / ms * 1e3:.1f} samples/s); CTA0 ran ~{evals:.0f} evals; instrumented cycles {tot/1e6:.1f} M ({tot/evals/1e3:.0f} k/eval)")
 for nm, v in zip(NAMES, prof):
     print(f"  {nm:34s} {v/1e6:10.2f} Mcyc  {100*v/tot:5.1f}%   {v/evals/1e3:8.1f} kcyc/eval")
+print(f"  evaluations on the canonical path (CTA 0): {int(prof[NFALLBACK])}")
